@@ -2,6 +2,7 @@
 """bench.py -- env-steps/s of the batched bsuite engine on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA engine
+    python bench.py ... --dump-outputs DIR                          # + the last timed step's outputs as DIR/*.npy
     python bench.py --impl reference [--steps K] [--warmup W]      # the reference's own step() loop on host cores
     torchrun --nproc-per-node N ... bench.py --gpus N ...           # one rank per GPU (weak scaling)
 
@@ -40,6 +41,9 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
   sys.path.insert(0, ROOT)
+# the tree may be read-only where the benchmark runs: no bytecode caches in it, from here or from the processes it starts
+sys.dont_write_bytecode = True
+os.environ['PYTHONDONTWRITEBYTECODE'] = '1'
 
 BSUITE_ID = 'deep_sea/11'          # size = 32, mapping_seed = 42
 SIZE = 32
@@ -389,6 +393,30 @@ def config_legs(args, rank, world, device, torch, dist, peak_gbs):
   return legs
 
 
+# ----------------------------------------------------------------------------- outputs of the timed path
+DUMP_OBSERVATION_LANES = 4096       # 4096 lanes x 32 x 32 float32 = 16.8 MB of the 268 MB observation tensor
+
+
+def dump_outputs(directory, last, summary, torch):
+  """Writes what the last timed step returned to its caller, as float32 / float64 .npy files: reward, discount and
+  step_type of every lane, the observations of a fixed seeded sample of lanes (sorted lane ids drawn by
+  RandomState(0)), and the log point's reduction of the Logging columns from the last window."""
+  import numpy as np
+  lanes = np.sort(np.random.RandomState(0).choice(BATCH_PER_GPU, DUMP_OBSERVATION_LANES, replace=False))
+  index = torch.as_tensor(lanes, device=last.observation.device)
+  arrays = {
+      'observation_sample': last.observation.index_select(0, index).cpu().numpy(),
+      'reward': last.reward.cpu().numpy(),
+      'discount': last.discount.cpu().numpy(),
+      'step_type': last.step_type.cpu().numpy().astype(np.float32),
+  }
+  if summary is not None:
+    arrays['log_point'] = summary.cpu().numpy().astype(np.float64)
+  os.makedirs(directory, exist_ok=True)
+  for name, array in arrays.items():
+    np.save(os.path.join(directory, name + '.npy'), array)
+
+
 # ----------------------------------------------------------------------------- engine arm
 def engine_main(args):
   import torch
@@ -453,7 +481,12 @@ def engine_main(args):
   if log_points is not None:
     for _ in range(2):                      # communicator set-up and first-use costs belong to the warm-up
       log_points.result(log_points.issue())
+  # keep_busy runs a wall-clock-dependent number of steps: the timed windows start from the state the warm-up left,
+  # so that the same arguments give the same inputs (and outputs) in every run
+  warm_state = env.state_dict()
   keep_busy(0.5)
+  torch.cuda.synchronize()
+  env.load_state_dict(warm_state)
   torch.cuda.synchronize()
 
   mid = max(1, K // 2)
@@ -484,6 +517,8 @@ def engine_main(args):
     total_ms = ev[0].elapsed_time(ev[4])
     step_ms = total_ms if log_points is None else ev[0].elapsed_time(ev[1]) + ev[2].elapsed_time(ev[3])
     windows.append((total_ms, step_ms))
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, ring[(K - 1) % RING], summary, torch)
   keep_busy(0.4)
   clocks = sampler.stop(load_t0 + 0.15, time.time()) if rank == 0 else None
   times = torch.tensor(windows, dtype=torch.float64, device=device)
@@ -774,7 +809,7 @@ def main():
   parser.add_argument('--skip-halves', action='store_true', help='skip the part-batches e2e legs')
   parser.add_argument('--e2e-parts', type=int, nargs='*', default=[2, 3, 4],
                       help='part counts of the part-batches e2e legs (rollouts.HostParts)')
-  parser.add_argument('--steps', type=int, default=400)
+  parser.add_argument('--steps', type=int, default=400, help='timed steps in each of the 5 windows of the headline value')
   parser.add_argument('--warmup', type=int, default=20)
   parser.add_argument('--impl', default='b200', choices=['b200', 'reference'])
   parser.add_argument('--skip-cpu-baseline', action='store_true')
@@ -785,8 +820,12 @@ def main():
   parser.add_argument('--skip-configs', action='store_true', help='skip the legs for BASELINE configs #3 / #4 / #5')
   parser.add_argument('--skip-traffic', action='store_true', help='do not re-measure DRAM traffic with ncu')
   parser.add_argument('--legs', default='catch_131072,cartpole_mc_262144,sweep_23x4096')
+  parser.add_argument('--dump-outputs', metavar='DIR', default=None,
+                      help='write the outputs of the last timed step to DIR/<name>.npy (rank 0)')
   parser.add_argument('--probe-traffic', action='store_true', help=argparse.SUPPRESS)
   args = parser.parse_args()
+  if args.steps < 1:
+    parser.error('--steps must be at least 1')
   if args.warmup < 3:
     args.warmup = 3
   if args.probe_traffic:

@@ -27,38 +27,15 @@ _SHIMS = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'shims')
 STREAM_ENV, STREAM_WRAPPER = 0, 1
 
 
-INSTALLED_ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), '_ref')
-_use_installed = False
-
-
 def reference_available() -> bool:
   return os.path.isdir(os.path.join(REFERENCE_ROOT, 'bsuite'))
 
 
-def installed_available() -> bool:
-  """oracle/_ref: the UNMODIFIED reference as `pip install --target` left it (oracle/install_ref.py); it travels to
-  the GPU box, where /root/reference does not exist."""
-  return os.path.isdir(os.path.join(INSTALLED_ROOT, 'bsuite'))
-
-
-def use_installed_reference() -> bool:
-  """Opt-in for a test that wants the live reference on a machine without /root/reference: from now on
-  `import_reference()` falls back to the installed copy.  `reference_available()` keeps meaning "the source tree is
-  here", so every other test behaves as before.  Returns whether a reference can be imported at all."""
-  global _use_installed  # pylint: disable=global-statement
-  if not reference_available() and installed_available():
-    _use_installed = True
-  return reference_available() or _use_installed
-
-
 def import_reference():
   """Imports and returns the reference's `bsuite` package (with shims for 4 absent pure-Python deps)."""
-  if reference_available():
-    root = REFERENCE_ROOT
-  elif _use_installed and installed_available():
-    root = INSTALLED_ROOT
-  else:
+  if not reference_available():
     raise RuntimeError(f'{REFERENCE_ROOT} is not present on this machine')
+  root = REFERENCE_ROOT
   repo_root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
   for path in (root, _SHIMS, repo_root):
     if path not in sys.path:

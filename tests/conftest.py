@@ -1,5 +1,6 @@
 """Test configuration: marker registration, library build check, shared helpers."""
 
+import functools
 import json
 import os
 import sys
@@ -12,7 +13,7 @@ if ROOT not in sys.path:
   sys.path.insert(0, ROOT)
 
 GOLDEN_DIR = os.path.join(ROOT, 'tests', 'golden')
-MNIST_DIR = os.path.join('/tmp', 'bsb_test_mnist')
+REFERENCE_DIR = os.path.join(GOLDEN_DIR, 'reference')
 
 
 def pytest_configure(config):
@@ -47,13 +48,14 @@ def _library_is_built():
 
 
 @pytest.fixture(scope='session')
-def mnist_dir():
+def mnist_dir(tmp_path_factory):
   """Synthetic idx-ubyte files identical to the ones oracle/gen_golden.py fed the reference."""
   from bsuite_b200 import datasets
   meta = dict(seed=0, num_train=256, num_test=16)
-  datasets.write_synthetic_mnist(MNIST_DIR, meta['num_train'], meta['num_test'], meta['seed'])
-  os.environ[datasets.ENV_VAR] = MNIST_DIR
-  return MNIST_DIR
+  path = str(tmp_path_factory.mktemp('mnist'))
+  datasets.write_synthetic_mnist(path, meta['num_train'], meta['num_test'], meta['seed'])
+  os.environ[datasets.ENV_VAR] = path
+  return path
 
 
 def golden_case_names():
@@ -64,6 +66,19 @@ def load_golden(name):
   data = np.load(os.path.join(GOLDEN_DIR, name + '.npz'))
   meta = json.loads(bytes(data['meta']).decode())
   return meta, data
+
+
+@functools.lru_cache(maxsize=None)
+def load_reference(name):
+  """What the unmodified reference returned for a test's inputs (tests/golden/reference/<name>.npz, recorded by
+  oracle/gen_reference_checks.py): arrays by key, the payloads of `.json` keys decoded."""
+  data = np.load(os.path.join(REFERENCE_DIR, name + '.npz'))
+  return {k: json.loads(bytes(data[k]).decode()) if k.endswith('.json') else data[k] for k in data.files}
+
+
+def none_nan(x):
+  """A timestep's reward or discount as the fixtures store it: None (FIRST) as NaN."""
+  return np.nan if x is None else float(x)
 
 
 # float-dynamics families: north_star tolerance 1e-6 (libm vs CUDA sin/cos/log differ in the last ulp)

@@ -6,7 +6,7 @@ import torch
 
 import bsuite_b200
 from bsuite_b200 import adapters
-from oracle import reference_runner as rr
+from tests import conftest as cf
 
 DEVICES = [pytest.param('cpu', id='host'), pytest.param('cuda', id='cuda', marks=pytest.mark.gpu)]
 
@@ -42,10 +42,8 @@ def test_small_state_tiling_matches_reference(size, shape):
   batched = adapters.to_image(shape, torch.as_tensor(np.stack([values, values * 2])).reshape(2, 1, size), batch_dims=1)
   np.testing.assert_array_equal(batched[0].numpy(), got)
   np.testing.assert_array_equal(batched[1].numpy(), got * 2)
-  if rr.reference_available():
-    rr.import_reference()
-    from bsuite.utils import wrappers  # pylint: disable=import-outside-toplevel
-    np.testing.assert_array_equal(got, wrappers.to_image(shape, values.reshape(1, size)))
+  want = cf.load_reference('to_image')[f'{size}/{"x".join(map(str, shape))}']     # the reference's wrappers.to_image
+  np.testing.assert_array_equal(got, want)
 
 
 def test_large_observations_need_skimage():

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 from tests import conftest as cf
@@ -42,9 +43,14 @@ def test_reference_arm_is_silent_on_other_ranks():
 
 
 @pytest.mark.gpu
-def test_engine_arm_prints_the_contract_line():
+def test_engine_arm_prints_the_contract_line(tmp_path):
   line = _run(['--steps', '40', '--warmup', '3', '--skip-cpu-baseline', '--skip-host-obs', '--skip-fused', '--skip-traffic',
-               '--legs', 'catch_131072'])
+               '--legs', 'catch_131072', '--dump-outputs', str(tmp_path)])
+  dumped = {name: np.load(tmp_path / name) for name in os.listdir(tmp_path)}
+  assert set(dumped) == {'observation_sample.npy', 'reward.npy', 'discount.npy', 'step_type.npy', 'log_point.npy'}
+  assert all(a.dtype in (np.float32, np.float64) for a in dumped.values())
+  assert sum(a.nbytes for a in dumped.values()) <= 64 << 20
+  assert dumped['reward.npy'].shape == (65536,) and dumped['observation_sample.npy'].shape[1:] == (32, 32)
   for key in COMMON + ('roofline', 'clocks'):
     assert key in line, key
   assert line['n_gpus'] == 1 and line['steps'] == 40 and line['scaling'] == 'weak' and line['data'] == 'synthetic'

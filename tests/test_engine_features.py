@@ -8,7 +8,7 @@ import torch
 
 import bsuite_b200
 from oracle import bsuite_oracle as oracle
-from oracle import reference_runner as rr
+from tests import conftest as cf
 
 DEVICES = [pytest.param('cpu', id='host'), pytest.param('cuda', id='cuda', marks=pytest.mark.gpu)]
 
@@ -95,18 +95,10 @@ def test_state_snapshot_restores_trajectory(device):
     other.load_state_dict(snapshot)
 
 
-class _Recorder:
-  def __init__(self):
-    self.rows = []
-
-  def write(self, data):
-    self.rows.append(dict(data))
-
-
 @pytest.mark.parametrize('device', DEVICES)
 def test_episode_stats_match_reference_logging_wrapper(device):
-  """The per-lane Logging accumulators (utils/wrappers.py:85-110) against the reference's own wrapper when it is
-  available, else against the same bookkeeping applied to the oracle trace."""
+  """The per-lane Logging accumulators (utils/wrappers.py:85-110) against the same bookkeeping applied to the oracle
+  trace, and against the rows the reference's own wrapper wrote (tests/golden/reference/final_logging_rows.npz)."""
   kwargs, seed, T, B = dict(rows=5, columns=3), 21, 90, 6
   env = bsuite_b200.make('catch', batch=B, device=device, seed=seed, reward_scale=30.0,
                          engine_kwargs=dict(reward_dtype='float64', track_episodes=True), **kwargs)
@@ -128,28 +120,20 @@ def test_episode_stats_match_reference_logging_wrapper(device):
         episode += 1
     got = [stats[k][lane] for k in ('steps', 'episode', 'total_return', 'episode_len', 'episode_return')]
     assert got == [steps, episode, total, ep_len, ep_ret]
-  if rr.reference_available():
-    # The reference's own Logging wrapper writes its row at LAST timesteps; compare the engine's columns at
-    # exactly such a moment (T2 chosen so that every lane's final call is a LAST: catch episodes are 5 calls).
-    rr.import_reference()
-    from bsuite.utils import wrappers  # pylint: disable=import-outside-toplevel
-    T2 = 85
-    env2 = bsuite_b200.make('catch', batch=B, device=device, seed=seed, reward_scale=30.0,
-                            engine_kwargs=dict(reward_dtype='float64', track_episodes=True), **kwargs)
-    ts = env2.rollout(T2, actions=torch.as_tensor(actions[:T2]))
-    assert np.all(_np(ts.step_type)[-1] == 2)
-    stats2 = {k: _np(v) for k, v in env2.episode_stats().items()}
-    for lane in range(B):
-      raw = rr.make_reference_env('catch', kwargs, 'philox', seed, lane, 'scale', 30.0)
-      raw.bsuite_num_episodes = 10**9
-      recorder = _Recorder()
-      logged = wrappers.Logging(raw, recorder, log_every=True)
-      for t in range(T2):
-        logged.step(int(actions[t, lane]))
-      final = recorder.rows[-1]
-      for key in ('steps', 'episode', 'total_return', 'episode_len', 'episode_return'):
-        assert final[key] == stats2[key][lane], key
-      assert final['total_regret'] == _np(env2.bsuite_info()['total_regret'])[lane]
+  # The reference's own Logging wrapper writes its row at LAST timesteps; compare the engine's columns at exactly
+  # such a moment (T2 chosen so that every lane's final call is a LAST: catch episodes are 5 calls).
+  T2 = 85
+  env2 = bsuite_b200.make('catch', batch=B, device=device, seed=seed, reward_scale=30.0,
+                          engine_kwargs=dict(reward_dtype='float64', track_episodes=True), **kwargs)
+  ts = env2.rollout(T2, actions=torch.as_tensor(actions[:T2]))
+  assert np.all(_np(ts.step_type)[-1] == 2)
+  stats2 = {k: _np(v) for k, v in env2.episode_stats().items()}
+  finals = cf.load_reference('final_logging_rows')['rows.json']
+  assert len(finals) == B
+  for lane, final in enumerate(finals):
+    for key in ('steps', 'episode', 'total_return', 'episode_len', 'episode_return'):
+      assert final[key] == stats2[key][lane], key
+    assert final['total_regret'] == _np(env2.bsuite_info()['total_regret'])[lane]
 
 
 @pytest.mark.parametrize('device', DEVICES)

@@ -1,6 +1,6 @@
 """INTEGRATION.md's reference-side binding, executed: `examples/reference_binding_stub.py` (plain ctypes, nothing
 from the bsuite_b200 package) reproduces the unmodified reference's deep_sea known answers -- digest, #LAST,
-bsuite_info -- and plugs into the reference's own registry when the reference is importable."""
+bsuite_info -- and, built the way the reference's own registry builds an environment, its traces."""
 
 import hashlib
 import importlib.util
@@ -11,7 +11,6 @@ import struct
 import numpy as np
 import pytest
 
-from oracle import reference_runner as rr
 from tests import conftest as cf
 
 
@@ -51,24 +50,14 @@ def test_stub_reproduces_reference_known_answers(row):
   env.close()
 
 
-@pytest.mark.skipif(not rr.reference_available(), reason='the reference tree is not present on this machine')
 def test_stub_registers_in_the_reference():
-  """bsuite.load_from_id('deep_sea/0') through the reference's OWN registry and sweep tables, with the stub class
-  swapped in for the numpy implementation: same trace as the reference's class."""
-  rr.import_reference()
-  import bsuite  # pylint: disable=import-outside-toplevel
-  from bsuite import bsuite as bsuite_registry  # pylint: disable=import-outside-toplevel
+  """The reference's registry builds an environment as EXPERIMENT_NAME_TO_ENVIRONMENT[name](**sweep.SETTINGS[id]);
+  the stub class built that way for 'deep_sea/2', with the reference's own settings for that id, gives the trace the
+  reference's class gave (tests/golden/reference/registry.npz)."""
+  ref = cf.load_reference('registry')
   stub = _stub()
-  original = bsuite_registry.EXPERIMENT_NAME_TO_ENVIRONMENT['deep_sea']
   actions = np.random.RandomState(3).randint(2, size=300)
-  want_env = bsuite.load_from_id('deep_sea/2')
-  want = [want_env.reset()] + [want_env.step(int(a)) for a in actions]
-  try:
-    bsuite_registry.EXPERIMENT_NAME_TO_ENVIRONMENT['deep_sea'] = (
-        lambda **kwargs: stub.DeepSeaB200(**kwargs))
-    env = bsuite.load_from_id('deep_sea/2')
-    assert isinstance(env, stub.DeepSeaB200)
-    got = [env.reset()] + [env.step(int(a)) for a in actions]
-  finally:
-    bsuite_registry.EXPERIMENT_NAME_TO_ENVIRONMENT['deep_sea'] = original
-  assert _digest(got) == _digest(want)
+  env = stub.DeepSeaB200(**ref['tables.json']['SETTINGS']['deep_sea/2'])
+  got = [env.reset()] + [env.step(int(a)) for a in actions]
+  env.close()
+  assert _digest(got) == ref['deep_sea_2_digest.json']

@@ -1,10 +1,9 @@
 """Pins oracle/bsuite_oracle.py (the CPU restatement) to the UNMODIFIED reference.
 
-The fixtures under tests/golden/ were recorded by oracle/gen_golden.py from
-/root/reference itself.  The oracle must reproduce every one of them exactly --
-including the float-dynamics families, since both run numpy/libm on the CPU --
-and the SURVEY.md 8c known-answer digests.  When /root/reference is present
-(this container) the oracle is additionally checked live against it.
+The fixtures under tests/golden/ were recorded by oracle/gen_golden.py and
+oracle/gen_reference_checks.py from the reference itself.  The oracle must
+reproduce every one of them exactly -- including the float-dynamics families,
+since both run numpy/libm on the CPU -- and the SURVEY.md 8c known-answer digests.
 """
 
 import hashlib
@@ -16,7 +15,6 @@ import numpy as np
 import pytest
 
 from oracle import bsuite_oracle as oracle
-from oracle import reference_runner as rr
 from tests import conftest as cf
 
 
@@ -87,7 +85,6 @@ def test_oracle_known_answer_digests(row):
   assert info == row['info']
 
 
-@pytest.mark.skipif(not rr.reference_available(), reason='/root/reference only exists in the build container')
 @pytest.mark.parametrize('env_class,kwargs,wrapper,arg', [
     ('deep_sea', dict(size=14, deterministic=False, mapping_seed=7), None, 0.),
     ('catch', dict(rows=6, columns=4), 'noise', 0.3),
@@ -96,15 +93,16 @@ def test_oracle_known_answer_digests(row):
     ('memory_chain', dict(memory_length=3, num_bits=5), None, 0.),
 ])
 def test_oracle_live_against_reference(env_class, kwargs, wrapper, arg):
-  """Fresh configurations (not among the committed fixtures), checked live where the reference exists."""
+  """Fresh configurations (not among the trace fixtures above): every call's timestep and the final bsuite_info()
+  against what the reference returned for them (tests/golden/reference/fresh_configurations.npz)."""
+  want = cf.load_reference('fresh_configurations')
   for rng, seed in (('philox', 99), ('mt19937', 3)):
-    ref = rr.make_reference_env(env_class, kwargs, rng, seed, lane=2, wrapper=wrapper, wrapper_arg=arg)
+    key = f'{env_class}/{rng}'
     env = oracle.OracleEnv(env_class, kwargs, rng=rng, seed=seed, lane=2, wrapper=wrapper, wrapper_arg=arg)
     actions = np.random.RandomState(1).randint(env.num_actions, size=400)
-    for a in actions:
-      ts = ref.step(int(a))
+    for t, a in enumerate(actions):
       st, r, d, o = env.step(int(a))
-      assert int(ts.step_type) == st
-      assert ts.reward == r and ts.discount == d
-      np.testing.assert_array_equal(np.asarray(ts.observation), o)
-    assert {k: float(v) for k, v in ref.bsuite_info().items()} == {k: float(v) for k, v in env.bsuite_info().items()}
+      assert want[f'{key}/step_type'][t] == st
+      np.testing.assert_array_equal([cf.none_nan(r), cf.none_nan(d)], [want[f'{key}/reward'][t], want[f'{key}/discount'][t]])
+      np.testing.assert_array_equal(want[f'{key}/observation'][t], o)
+    assert want[f'{key}/info.json'] == {k: float(v) for k, v in env.bsuite_info().items()}

@@ -110,31 +110,31 @@ def test_cuda_matches_oracle_on_random_configurations(chunk):
     _check(_draw_case(rng), 'cuda')
 
 
-from oracle import reference_runner as rr  # noqa: E402
-
-
-@pytest.mark.skipif(not rr.reference_available(), reason='/root/reference only exists in the build container')
 @pytest.mark.parametrize('chunk', range(4))
 def test_oracle_matches_live_reference_on_random_configurations(chunk):
-  """Widens the oracle's pin beyond the committed fixtures: the same random configuration generator, oracle vs the
-  UNMODIFIED reference, lane by lane (exact, float families included: both are numpy/libm on this CPU)."""
+  """Widens the oracle's pin beyond the trace fixtures: the same random configuration generator, oracle vs what the
+  UNMODIFIED reference returned for each drawn case, lane by lane (tests/golden/reference/random_configurations.npz,
+  observations by digest; exact, float families included: both are numpy/libm on the CPU)."""
+  from oracle.gen_reference_checks import observation_digest
+  recorded = cf.load_reference('random_configurations')[f'chunk_{chunk}.json']
   rng = np.random.RandomState(9000 + chunk)
-  for _ in range(25):
+  for want in recorded:
     case = _draw_case(rng)
+    assert case == want['case']
     seed = case['seed'] % (2**32 - 10**6 - 100) if case['rng'] == 'mt19937' else case['seed']
     T = case['steps']
     lanes = min(case['batch'], 3)
-    for lane in range(lanes):
-      ref = rr.make_reference_env(case['family'], case['kwargs'], case['rng'], seed, case['offset'] + lane,
-                                  case['wrapper'], case['arg'])
+    assert len(want['lanes']) == lanes
+    for lane, ref in enumerate(want['lanes']):
       env = oracle.OracleEnv(case['family'], case['kwargs'], rng=case['rng'], seed=seed, lane=case['offset'] + lane,
                              wrapper=case['wrapper'], wrapper_arg=case['arg'])
       actions = np.random.RandomState(lane).randint(env.num_actions, size=T)
+      observations = []
       for t, a in enumerate(actions):
-        if t in case['reset_at']:
-          ts, (st, r, d, o) = ref.reset(), env.reset()
-        else:
-          ts, (st, r, d, o) = ref.step(int(a)), env.step(int(a))
-        assert int(ts.step_type) == st and ts.reward == r and ts.discount == d, case
-        np.testing.assert_array_equal(np.asarray(ts.observation), o, err_msg=str(case))
-      assert {k: float(v) for k, v in ref.bsuite_info().items()} == {k: float(v) for k, v in env.bsuite_info().items()}
+        st, r, d, o = env.reset() if t in case['reset_at'] else env.step(int(a))
+        assert ref['step_type'][t] == st, case
+        np.testing.assert_array_equal([cf.none_nan(r), cf.none_nan(d)], [ref['reward'][t], ref['discount'][t]],
+                                      err_msg=str(case))
+        observations.append(np.asarray(o, np.float32))
+      assert observation_digest(np.stack(observations)) == ref['observation_sha256'], case
+      assert ref['info'] == {k: float(v) for k, v in env.bsuite_info().items()}

@@ -1,13 +1,15 @@
 """Recorder / CsvLogger: the Logging bookkeeping pinned by the reference's utils/wrappers_test.py:84-121, the log
 schedule of wrappers.py:140-147, and CSV files the reference's own csv_load can read."""
 
+import os
+
 import numpy as np
 import pytest
 
 import bsuite_b200
 from bsuite_b200 import dm_env
 from bsuite_b200 import recording
-from oracle import reference_runner as rr
+from tests import conftest as cf
 
 
 class _Cycle(dm_env.Environment):
@@ -86,33 +88,28 @@ def test_csv_recorder_round_trip(tmp_path):
     bsuite_b200.load_and_record('catch/3', str(tmp_path), logging_mode='sqlite', device='cpu')
 
 
-@pytest.mark.skipif(not rr.reference_available(), reason='/root/reference only exists in the build container')
 def test_reference_csv_load_reads_our_files(tmp_path):
-  """Same seed, same actions -> the reference's Logging + csv_logging and ours write identical tables, and the
-  reference's csv_load.load_bsuite parses ours."""
-  bsuite = rr.import_reference()
-  from bsuite.logging import csv_load, csv_logging  # pylint: disable=import-outside-toplevel
-  from bsuite.environments import catch as ref_catch  # pylint: disable=import-outside-toplevel
-  ours_dir, ref_dir = str(tmp_path / 'ours'), str(tmp_path / 'ref')
+  """Same seed, same actions -> ours writes the file the reference's Logging + csv_logging wrote (same name, same
+  bytes; tests/golden/reference/recording.npz), so the reference's csv_load.load_bsuite parses ours as its own."""
+  want = cf.load_reference('recording')['csv/catch_seed_5.json']
+  ours_dir = str(tmp_path / 'ours')
   ours = recording.Recorder(bsuite_b200.make('catch', device='cpu', seed=5),
                             recording.CsvLogger('catch/0', ours_dir))
-  ref = csv_logging.wrap_environment(ref_catch.Catch(seed=5), 'catch/0', ref_dir)
-  rng = np.random.RandomState(1)
+  rng, rewards = np.random.RandomState(1), []
   for _ in range(30):
-    a, b = ours.reset(), ref.reset()
+    a = ours.reset()
     while not a.last():
-      action = int(rng.randint(3))
-      a, b = ours.step(action), ref.step(action)
-      assert a.reward == b.reward
-  df_ours, _ = csv_load.load_bsuite(ours_dir)
-  df_ref, _ = csv_load.load_bsuite(ref_dir)
-  columns = ['steps', 'episode', 'total_return', 'episode_len', 'episode_return', 'total_regret', 'bsuite_id']
-  assert df_ours[columns].reset_index(drop=True).equals(df_ref[columns].reset_index(drop=True))
+      a = ours.step(int(rng.randint(3)))
+      rewards.append(a.reward)
+  assert rewards == want['rewards']
+  assert os.listdir(ours_dir) == [want['file_name']]
+  with open(os.path.join(ours_dir, want['file_name'])) as fh:
+    assert fh.read() == want['text']
 
 
 def test_terminal_logger_formats_like_the_reference():
   """`k1 = v1 | k2 = v2`, keys sorted, integers plain, other numbers with 4 decimals (terminal_logging.py:57-74);
-  compared with the reference's own formatter when it is importable."""
+  compared with the line the reference's own formatter made of the same dict."""
   data = {'steps': 12, 'total_return': -3.0, 'episode': np.int64(4), 'episode_return': np.float64(0.123456),
           'name': 'catch/0', 'flag': True}
   lines = []
@@ -121,10 +118,7 @@ def test_terminal_logger_formats_like_the_reference():
   raw = []
   recording.TerminalLogger(pretty_print=False, print_fn=raw.append).write(data)
   assert raw == [data]
-  if rr.reference_available():
-    rr.import_reference()
-    from bsuite.logging import terminal_logging  # pylint: disable=import-outside-toplevel
-    assert terminal_logging.pretty_dict(data) == lines[0]
+  assert cf.load_reference('recording')['terminal/pretty_dict.json'] == lines[0]
 
 
 def test_load_and_record_modes(tmp_path, capsys):
@@ -152,45 +146,19 @@ _BATCHED_DEVICES = [pytest.param('cpu', id='host'),
                     pytest.param('cuda', id='cuda', marks=[pytest.mark.gpu, pytest.mark.runs_last])]
 
 
-def _need_reference(device, request):
-  """The reference's source tree (build container), or -- for the CUDA variants on the GPU box, which has no tree --
-  the unmodified reference as installed under oracle/_ref.  That combination has not run anywhere yet (the container
-  has no GPU, the round's GPU budget was spent before it existed): non-strict xfail, scheduled last."""
-  if rr.reference_available():
-    return
-  if device == 'cuda' and rr.use_installed_reference():
-    request.applymarker(pytest.mark.xfail(strict=False, reason='first run on a GPU with the installed reference: reported, not gating'))
-    return
-  pytest.skip('needs the reference (source tree, or oracle/_ref for the CUDA variants)')
-
-
-def _reference_rows(env_class, kwargs, seed, lane, actions, wrapper=None, arg=None):
-  """Rows the reference's own Logging wrapper writes for one lane (utils/wrappers.py:85-125)."""
-  rr.import_reference()
-  from bsuite.utils import wrappers  # pylint: disable=import-outside-toplevel
-
-  class Rows:
-    def __init__(self):
-      self.rows = []
-
-    def write(self, data):
-      self.rows.append(dict(data))
-
-  raw = rr.make_reference_env(env_class, kwargs, 'philox', seed, lane, wrapper, arg)
-  raw.bsuite_num_episodes = 10000
-  sink = Rows()
-  logged = wrappers.Logging(raw, sink)
-  for a in actions:
-    logged.step(int(a))
-  return sink.rows
+def _reference_rows(bsuite_id, lane):
+  """Rows the reference's own Logging wrapper wrote for one lane (utils/wrappers.py:85-125), recorded with the
+  same seed and actions as the tests below (tests/golden/reference/recording.npz)."""
+  ref = cf.load_reference('recording')
+  columns = ref[f'{bsuite_id}/columns.json']
+  return [dict(zip(columns, row)) for row in ref[f'{bsuite_id}/rows'][lane, :ref[f'{bsuite_id}/counts'][lane]].tolist()]
 
 
 @pytest.mark.parametrize('device', _BATCHED_DEVICES)
-def test_batched_log_rows_equal_the_reference_logging_wrapper_row_for_row(device, tmp_path, request):
+def test_batched_log_rows_equal_the_reference_logging_wrapper_row_for_row(device, tmp_path):
   """VERDICT r01 item 8: 64 lanes x 1 000 episodes of catch.  Every lane's rows, recorded on the device at the
-  log-spaced episode counts, equal the rows the reference wrapper writes for the same lane -- and the CSV files
-  written from them load with the reference's csv_load."""
-  _need_reference(device, request)
+  log-spaced episode counts, equal the rows the reference wrapper writes for the same lane -- and the CSV file
+  written from a lane's rows is the one the reference's csv_logging writes for it, byte for byte."""
   import torch
   B, episodes = 64, 1000
   T = episodes * 10                                 # catch: 9 transitions + the auto-reset call per episode
@@ -204,16 +172,16 @@ def test_batched_log_rows_equal_the_reference_logging_wrapper_row_for_row(device
   assert list(logged['columns']) == ['steps', 'episode', 'total_return', 'episode_len', 'episode_return', 'total_regret']
   assert (counts == 36).all()                       # 1, 2, ..., 10, 12, ..., 1000: 10 + 13 + 13 rows
   for lane in range(B):
-    want = _reference_rows('catch', {}, 11, lane, actions[:, lane])
+    want = _reference_rows('catch/0', lane)
     assert len(want) == counts[lane]
     for k, row in enumerate(want):
       got = dict(zip(logged['columns'], rows[k, :, lane]))
       assert {c: float(v) for c, v in row.items()} == got, (lane, k)
-  from bsuite.logging import csv_load  # pylint: disable=import-outside-toplevel
   dirs = recording.write_lane_csvs(env, 'catch/0', str(tmp_path), lanes=range(4))
-  df, _ = csv_load.load_bsuite(dirs[2])
-  assert list(df['episode']) == list(logged['schedule'][:36]) and set(df['bsuite_id']) == {'catch/0'}
-  assert list(df['total_regret']) == [r['total_regret'] for r in _reference_rows('catch', {}, 11, 2, actions[:, 2])]
+  want = cf.load_reference('recording')['catch/0/lane_2_csv.json']
+  assert os.listdir(dirs[2]) == [want['file_name']]
+  with open(os.path.join(dirs[2], want['file_name'])) as fh:
+    assert fh.read() == want['text']
   with pytest.raises(ValueError, match='already exists'):
     recording.write_lane_csvs(env, 'catch/0', str(tmp_path), lanes=range(2))
 
@@ -224,20 +192,18 @@ def test_batched_log_rows_equal_the_reference_logging_wrapper_row_for_row(device
     ('deep_sea_stochastic/0', 'deep_sea', dict(size=10, deterministic=False, mapping_seed=42), 2, None, None),
     ('bandit_scale/3', 'bandit', dict(mapping_seed=3), 11, 'scale', 1.0),
 ])
-def test_batched_log_rows_for_other_families(device, bsuite_id, env_class, kwargs, n_act, wrapper, arg, request):
-  _need_reference(device, request)
+def test_batched_log_rows_for_other_families(device, bsuite_id, env_class, kwargs, n_act, wrapper, arg):
+  """The reference rows were recorded from `env_class(**kwargs)` with `wrapper` (reward_scale from the sweep
+  settings), seed 2, on the same actions."""
   import torch
-  from bsuite_b200 import sweep
   B, T = 6, 3000
   env = bsuite_b200.load_from_id(bsuite_id, batch=B, device=device, seed=2, record_rows=True)
-  settings = dict(sweep.SETTINGS[bsuite_id])
-  arg = settings.get('reward_scale', arg)
   actions = np.random.RandomState(9).randint(n_act, size=(T, B)).astype(np.int32)
   env.rollout(T, actions=torch.as_tensor(actions))
   logged = env.logged_rows()
   rows, counts = logged['rows'].cpu().numpy(), logged['counts'].cpu().numpy()
   for lane in range(B):
-    want = _reference_rows(env_class, kwargs, 2, lane, actions[:, lane], wrapper, arg)
+    want = _reference_rows(bsuite_id, lane)
     assert len(want) == counts[lane] > 0
     for k, row in enumerate(want):
       for c, v in row.items():
@@ -246,18 +212,13 @@ def test_batched_log_rows_for_other_families(device, bsuite_id, env_class, kwarg
 
 
 # ---------------------------------------------------------------------------- CUDA rows against the host path's rows
-# The tests above compare the device-side recorder with the reference's own Logging wrapper, which needs the
-# reference tree: in the build container that pins the HOST path (no GPU there), and on the GPU box (no reference
-# tree there) their CUDA variants are skipped.  These close the chain on the GPU box without the reference: the same
-# `__host__ __device__` recorder on CUDA against the engine's host path, which the tests above pin to the reference.
-# They were written after the round's GPU budget was spent and have not run on a GPU yet: non-strict xfail (an XPASS
-# is the verification, a failure is reported without gating the suite) and scheduled last.
-_FIRST_GPU_RUN = pytest.mark.xfail(strict=False, reason='first run on a GPU: reported, not gating (see the comment above)')
+# The tests above compare the device-side recorder with the rows the reference's own Logging wrapper wrote; these
+# compare the same `__host__ __device__` recorder on CUDA with the engine's host path over more configurations and
+# call patterns (two-phase host steps, mid-episode resets).
 
 
 @pytest.mark.gpu
 @pytest.mark.runs_last
-@_FIRST_GPU_RUN
 @pytest.mark.parametrize('bsuite_id,batch,steps', [('catch/0', 64, 10000), ('cartpole/0', 6, 3000),
                                                    ('deep_sea_stochastic/0', 6, 3000), ('bandit_scale/3', 6, 3000),
                                                    ('deep_sea/11', 70, 4000)])
@@ -289,7 +250,6 @@ def test_device_log_rows_equal_the_host_path_rows(bsuite_id, batch, steps):
 
 @pytest.mark.gpu
 @pytest.mark.runs_last
-@_FIRST_GPU_RUN
 def test_device_log_rows_through_host_driven_steps_equal_the_host_path_rows():
   """The two-phase host step (deep_sea N = 32: transitions first, rows written from its phase 1) records the same rows."""
   import torch
@@ -312,7 +272,6 @@ def test_device_log_rows_through_host_driven_steps_equal_the_host_path_rows():
 
 @pytest.mark.gpu
 @pytest.mark.runs_last
-@_FIRST_GPU_RUN
 def test_device_episode_stats_across_mid_episode_resets_equal_the_host_path():
   """tests/test_round2_features.py pins the Logging columns across explicit mid-episode reset() calls to the reference's
   wrapper on the host path (its CUDA variant needs the reference tree); here CUDA against that host path, after

@@ -7,7 +7,7 @@ import torch
 import bsuite_b200
 from bsuite_b200 import rollouts
 from oracle import bsuite_oracle as oracle
-from oracle import reference_runner as rr
+from tests import conftest as cf
 
 DEVICES = [pytest.param('cpu', id='host'), pytest.param('cuda', id='cuda', marks=pytest.mark.gpu)]
 
@@ -38,19 +38,20 @@ def test_batched_run_loop_with_random_agent(device):
   assert abs(mean_return - 0.5) < 0.02          # uniform policy over rewards linspace(0, 1, 11)
 
 
-@pytest.mark.skipif(not rr.reference_available(), reason='/root/reference only exists in the build container')
 def test_reference_experiment_loop_runs_unmodified_on_the_adapter():
-  """bsuite/baselines/experiment.run + baselines/random/agent.Random, imported from the reference, drive our B = 1
-  environment exactly as they drive the reference's (same seed -> same episode returns)."""
-  rr.import_reference()
-  from bsuite.baselines import experiment  # pylint: disable=import-outside-toplevel
-  from bsuite.baselines.random import agent as random_agent  # pylint: disable=import-outside-toplevel
-  from bsuite.environments import catch as ref_catch  # pylint: disable=import-outside-toplevel
+  """bsuite/baselines/experiment.run + baselines/random/agent.Random(seed=2) on the reference's catch(seed=9): the
+  actions that loop took, episode by episode, drive our B = 1 environment through the same reset() / step() calls to
+  the same episode ends and the same returns (tests/golden/reference/experiment_loop.npz)."""
+  ref = cf.load_reference('experiment_loop')
   ours = bsuite_b200.make('catch', device='cpu', seed=9)
-  theirs = ref_catch.Catch(seed=9)
-  experiment.run(random_agent.Random(ours.action_spec(), seed=2), ours, num_episodes=40)
-  experiment.run(random_agent.Random(theirs.action_spec(), seed=2), theirs, num_episodes=40)
-  assert ours.bsuite_info() == theirs.bsuite_info()
+  assert len(ref['episodes.json']) == 40
+  for actions in ref['episodes.json']:
+    ts = ours.reset()
+    for t, action in enumerate(actions):
+      assert not ts.last()
+      ts = ours.step(action)
+      assert ts.last() == (t == len(actions) - 1)
+  assert {k: float(v) for k, v in ours.bsuite_info().items()} == ref['info.json']
 
 
 def test_replay_ring_matches_the_reference_semantics():

@@ -9,7 +9,6 @@ import torch
 
 import bsuite_b200
 from bsuite_b200 import _lib
-from oracle import reference_runner as rr
 
 from tests import conftest as cf
 
@@ -73,50 +72,34 @@ def test_device_actions_out_of_range_are_clamped_and_flagged(bsuite_id, mnist_di
 
 
 # ---------------------------------------------------------------------------- Logging bookkeeping vs the reference
-class _Rows:
-  def __init__(self):
-    self.rows = []
-
-  def write(self, data):
-    self.rows.append(dict(data))
-
-
 @pytest.mark.parametrize('device', DEVICES)
 def test_episode_stats_follow_the_reference_wrapper_across_mid_episode_resets(device):
   """utils/wrappers.py:85-110 zeroes episode_len / episode_return after a LAST only: an explicit reset() in the
-  middle of an episode leaves them running.  Columns are compared at every LAST (when the reference writes)."""
-  if not rr.reference_available():
-    pytest.skip('needs /root/reference')
-  rr.import_reference()
-  from bsuite.utils import wrappers  # pylint: disable=import-outside-toplevel
+  middle of an episode leaves them running.  Columns are compared at every LAST (when the reference writes) with the
+  rows the reference's wrapper (log_every) wrote for the same seed and script (tests/golden/reference/
+  mid_episode_resets.npz)."""
+  ref = cf.load_reference('mid_episode_resets')
   kwargs, seed, B = dict(rows=6, columns=3), 5, 4
   env = bsuite_b200.make('catch', batch=B, device=device, seed=seed,
                          engine_kwargs=dict(reward_dtype='float64', track_episodes=True), **kwargs)
-  refs, recorders = [], []
-  for lane in range(B):
-    raw = rr.make_reference_env('catch', kwargs, 'philox', seed, lane)
-    raw.bsuite_num_episodes = 10**9
-    recorders.append(_Rows())
-    refs.append(wrappers.Logging(raw, recorders[-1], log_every=True))
   rng = np.random.RandomState(0)
   script = ['reset'] + ['step'] * 3 + ['reset'] + ['step'] * 7 + ['reset', 'reset'] + ['step'] * 11 + ['reset'] + ['step'] * 9
-  for op in script:
+  assert script == ref['script.json']
+  for i, op in enumerate(script):
     if op == 'reset':
       ts = env.reset()
-      for ref in refs:
-        ref.reset()
     else:
       actions = rng.randint(3, size=B).astype(np.int32)
       ts = env.step(torch.as_tensor(actions))
-      for lane, ref in enumerate(refs):
-        ref.step(int(actions[lane]))
     stats = {k: _np(v) for k, v in env.episode_stats().items()}
     for lane in range(B):
-      if int(_np(ts.step_type)[lane]) == 2:             # the reference has just written a row for this lane
-        row = recorders[lane].rows[-1]
-        for key in ('steps', 'episode', 'total_return', 'episode_len', 'episode_return'):
-          assert row[key] == stats[key][lane], (op, lane, key)
-  assert sum(len(r.rows) for r in recorders) >= 8
+      wrote = ref['counts'][i, lane] > (ref['counts'][i - 1, lane] if i else 0)
+      assert wrote == (int(_np(ts.step_type)[lane]) == 2), (op, lane)
+      if wrote:                                          # the reference has just written a row for this lane
+        row = ref['last_row'][i, lane]
+        for k, key in enumerate(('steps', 'episode', 'total_return', 'episode_len', 'episode_return')):
+          assert row[k] == stats[key][lane], (op, lane, key)
+  assert ref['counts'][-1].sum() >= 8
 
 
 # ---------------------------------------------------------------------------- snapshots and seeds

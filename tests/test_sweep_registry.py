@@ -1,11 +1,12 @@
 """The experiment registry: ids, kwargs, episodes and tags equal the reference's bsuite/sweep.py."""
 
+import numpy as np
 import pytest
 
 import bsuite_b200
 from bsuite_b200 import experiments
 from bsuite_b200 import sweep
-from oracle import reference_runner as rr
+from tests import conftest as cf
 
 
 def test_census():
@@ -38,39 +39,34 @@ def test_id_parsing():
       bsuite_b200.unpack_bsuite_id(bad)
 
 
-@pytest.mark.skipif(not rr.reference_available(), reason='/root/reference only exists in the build container')
 def test_registry_equals_reference():
-  bsuite = rr.import_reference()
-  from bsuite import sweep as ref  # pylint: disable=import-outside-toplevel
-  assert tuple(ref.SWEEP) == sweep.SWEEP
-  assert tuple(ref.TESTING) == sweep.TESTING
-  assert {k: dict(v) for k, v in ref.SETTINGS.items()} == {k: dict(v) for k, v in sweep.SETTINGS.items()}
-  assert dict(ref.EPISODES) == dict(sweep.EPISODES)
-  assert {k: tuple(v) for k, v in ref.TAGS.items()} == dict(sweep.TAGS)
-  assert set(bsuite.bsuite.EXPERIMENT_NAME_TO_ENVIRONMENT) == set(bsuite_b200.EXPERIMENT_NAME_TO_ENVIRONMENT)
+  """Against the reference's sweep tables and registry keys (tests/golden/reference/registry.npz)."""
+  ref = cf.load_reference('registry')['tables.json']
+  assert tuple(ref['SWEEP']) == sweep.SWEEP
+  assert tuple(ref['TESTING']) == sweep.TESTING
+  assert ref['SETTINGS'] == {k: dict(v) for k, v in sweep.SETTINGS.items()}
+  assert ref['EPISODES'] == dict(sweep.EPISODES)
+  assert {k: tuple(v) for k, v in ref['TAGS'].items()} == dict(sweep.TAGS)
+  assert set(ref['EXPERIMENT_NAME_TO_ENVIRONMENT']) == set(bsuite_b200.EXPERIMENT_NAME_TO_ENVIRONMENT)
   for name in ('BANDIT', 'CARTPOLE_SWINGUP', 'DEEP_SEA_STOCHASTIC', 'UMBRELLA_LENGTH'):
-    assert getattr(ref, name) == getattr(sweep, name)
+    assert tuple(ref[name]) == tuple(getattr(sweep, name))
 
 
-@pytest.mark.skipif(not rr.reference_available(), reason='/root/reference only exists in the build container')
 def test_every_setting_loads_with_reference_specs(mnist_dir):
   """One id per (experiment, distinct kwargs set) -- bsuite/tests/environments_test.py:25-49 -- on the host path;
-  specs and bsuite_num_episodes must equal the reference environment's."""
-  bsuite = rr.import_reference()
-  from bsuite.utils import datasets as ref_datasets  # pylint: disable=import-outside-toplevel
-  original = ref_datasets.load_mnist
-  ref_datasets.load_mnist = lambda directory=mnist_dir: original(directory)
-  try:
-    for name, ids in sweep.BY_EXPERIMENT.items():
-      for bsuite_id in (ids[0], ids[-1]):
-        env = bsuite_b200.load_from_id(bsuite_id, device='cpu')
-        ref = bsuite.load_from_id(bsuite_id)
-        assert env.bsuite_num_episodes == ref.bsuite_num_episodes, bsuite_id
-        a, b = env.action_spec(), ref.action_spec()
-        assert (a.num_values, a.dtype, a.name) == (b.num_values, b.dtype, b.name), bsuite_id
-        a, b = env.observation_spec(), ref.observation_spec()
-        assert (a.shape, a.dtype, a.name, type(a).__name__) == (b.shape, b.dtype, b.name, type(b).__name__), bsuite_id
-        assert set(env.bsuite_info()) == set(ref.bsuite_info()), bsuite_id
-        env.close()
-  finally:
-    ref_datasets.load_mnist = original
+  specs and bsuite_num_episodes must equal the reference environment's (tests/golden/reference/registry.npz)."""
+  want = cf.load_reference('registry')['specs.json']
+  checked = set()
+  for ids in sweep.BY_EXPERIMENT.values():
+    for bsuite_id in (ids[0], ids[-1]):
+      env = bsuite_b200.load_from_id(bsuite_id, device='cpu')
+      ref = want[bsuite_id]
+      assert env.bsuite_num_episodes == ref['bsuite_num_episodes'], bsuite_id
+      a = env.action_spec()
+      assert [int(a.num_values), str(np.dtype(a.dtype)), a.name] == ref['action'], bsuite_id
+      a = env.observation_spec()
+      assert [list(a.shape), str(np.dtype(a.dtype)), a.name, type(a).__name__] == ref['observation'], bsuite_id
+      assert sorted(env.bsuite_info()) == ref['info'], bsuite_id
+      env.close()
+      checked.add(bsuite_id)
+  assert checked == set(want)
