@@ -8,6 +8,8 @@ Public surface (mirrors `bsuite/__init__.py:18-24` and `bsuite/bsuite.py`):
   make(environment_class, batch=..., **kwargs) -> construct a raw environment class
   sweep                                        -> SETTINGS / SWEEP / TAGS / TESTING / EPISODES
   EXPERIMENT_NAME_TO_ENVIRONMENT               -> experiment name -> loader
+  SweepBatch(ids, lanes=B, record_rows=True)   -> many bsuite_ids at once; .scores() per lane
+  Scorer(envs_by_id).run()                     -> per-lane scores / finished / tag averages (scoring)
 
 The compute lives in `libbsuite_b200.so` (hand-written sm_100a CUDA behind the C
 ABI of include/bsuite_b200.h); importing this package does not load it, creating
@@ -34,5 +36,8 @@ from bsuite_b200.registry import (  # noqa: E402,F401
     unpack_bsuite_id,
 )
 from bsuite_b200.environment import BatchedEnvironment, DmEnvAdapter, StepBuffers  # noqa: E402,F401
+from bsuite_b200 import scoring  # noqa: E402,F401
+from bsuite_b200.scoring import Scorer  # noqa: E402,F401
+from bsuite_b200.suite import SweepBatch  # noqa: E402,F401
 
 __version__ = '0.1.0'

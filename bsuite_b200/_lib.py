@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # BSB_LIBRARY points the binding at another build of the SAME library (tools/host_sanitize.sh: ASan/UBSan build)
 LIB_PATH = os.environ.get('BSB_LIBRARY') or os.path.join(_HERE, 'libbsuite_b200.so')
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 DEVICE_HOST = -1
 MAX_INFO = 4
 COMM_ID_BYTES = 128
@@ -60,6 +60,18 @@ class Outputs(ctypes.Structure):
               ('discount', ctypes.c_void_p), ('step_type', ctypes.c_void_p)]
 
 
+class ScoreSource(ctypes.Structure):
+  """struct bsb_score_source."""
+  _fields_ = [('experiment', ctypes.c_int32), ('device', ctypes.c_int32), ('batch', ctypes.c_int64),
+              ('n_points', ctypes.c_int32), ('n_columns', ctypes.c_int32),
+              ('col_episode', ctypes.c_int32), ('col_value', ctypes.c_int32), ('col_best', ctypes.c_int32),
+              ('reserved0', ctypes.c_int32), ('group_key', ctypes.c_double),
+              ('rows', ctypes.c_void_p), ('counts', ctypes.c_void_p)]
+
+
+NUM_EXPERIMENTS, NUM_TAGS = 23, 7
+
+
 EXPORTS = {
     # name: (restype, argtypes)
     'bsb_abi_version': (ctypes.c_int32, []),
@@ -104,6 +116,15 @@ EXPORTS = {
     'bsb_log_point': (ctypes.c_int32, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_void_p), ctypes.c_int32, ctypes.c_void_p,
                                        ctypes.c_void_p, ctypes.c_void_p]),
     'bsb_comm_wait': (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p]),
+    'bsb_experiment_name': (ctypes.c_char_p, [ctypes.c_int32]),
+    'bsb_tag_name': (ctypes.c_char_p, [ctypes.c_int32]),
+    'bsb_score_source_from_env': (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_double,
+                                                   ctypes.POINTER(ScoreSource)]),
+    'bsb_scorer_create': (ctypes.c_int32, [ctypes.POINTER(ScoreSource), ctypes.c_int32, ctypes.c_int64, ctypes.c_int32,
+                                           ctypes.POINTER(ctypes.c_void_p)]),
+    'bsb_scorer_run': (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                        ctypes.c_void_p]),
+    'bsb_scorer_destroy': (ctypes.c_int32, [ctypes.c_void_p]),
     'bsb_launch_count': (ctypes.c_int64, []),
 }
 

@@ -17,9 +17,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 FAMILIES = ('deep_sea', 'catch', 'cartpole', 'cartpole_swingup', 'mountain_car', 'memory_chain', 'bandit',
             'umbrella_chain', 'discounting_chain', 'mnist')
-SOURCES = [os.path.join(CSRC, 'bsb_engine.cu'), os.path.join(CSRC, 'bsb_comm.cu')] + [os.path.join(CSRC, f'fam_{name}.cu') for name in FAMILIES]
+SOURCES = [os.path.join(CSRC, 'bsb_engine.cu'), os.path.join(CSRC, 'bsb_comm.cu'), os.path.join(CSRC, 'bsb_scoring.cu')] + [os.path.join(CSRC, f'fam_{name}.cu') for name in FAMILIES]
 HEADERS = [os.path.join(CSRC, f) for f in ('bsb_rng.cuh', 'bsb_families.cuh', 'bsb_kernels.cuh', 'bsb_env.h',
-                                           'bsb_dispatch.cuh')] + [
+                                           'bsb_dispatch.cuh', 'bsb_scoring.cuh')] + [
     os.path.join(os.path.dirname(HERE), 'include', 'bsuite_b200.h')]
 OUTPUT = os.path.join(HERE, 'libbsuite_b200.so')
 OBJ_DIR = os.path.join(HERE, 'build')

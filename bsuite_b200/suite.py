@@ -48,7 +48,7 @@ class GraphedSweep:
 class SweepBatch:
 
   def __init__(self, bsuite_ids: Optional[Sequence[str]] = None, lanes: int = 4096, device='cuda', seed: int = 0,
-               rank: int = 0, world: int = 1, track_episodes: bool = True, ring: int = 1):
+               rank: int = 0, world: int = 1, track_episodes: bool = True, ring: int = 1, record_rows: bool = False):
     import torch
     self._torch = torch
     self.bsuite_ids = list(bsuite_ids) if bsuite_ids is not None else one_per_experiment()
@@ -56,7 +56,7 @@ class SweepBatch:
     self.lanes, self.local_lanes, self.lane_offset = lanes, count, first
     self.envs = {
         bsuite_id: registry.load_from_id(bsuite_id, batch=count, device=device, seed=seed, lane_offset=first,
-                                         track_episodes=track_episodes)
+                                         track_episodes=track_episodes, record_rows=record_rows)
         for bsuite_id in self.bsuite_ids
     }
     self._device = next(iter(self.envs.values())).device
@@ -68,6 +68,8 @@ class SweepBatch:
     self._buffer_steps = None
     self._lp = None
     self._cols = None
+    self.record_rows = bool(record_rows)
+    self._scorer = None
 
   def _ensure_buffers(self, num_steps: int):
     if self._buffer_steps != num_steps:
@@ -166,11 +168,26 @@ class SweepBatch:
     """The one collective of the path, synchronous form: returns [world, n_ids, 3] (see `issue_log_point`)."""
     return self.log_point_result(self.issue_log_point())
 
+  def scores(self, out=None):
+    """Per-lane bsuite scores of this rank's lanes (`record_rows=True`): dict(scores=[23, local_lanes],
+    finished=[23, local_lanes], tags=[7, local_lanes]) on the batch's device, computed by one kernel launch on the
+    current stream from the rows recorded so far (`scoring.Scorer`).  Lanes are independent runs, so a rank needs
+    no collective to score; a caller that wants the whole population gathers these blocks itself."""
+    if not self.record_rows:
+      raise RuntimeError('SweepBatch.scores() needs the rows of every lane: create the SweepBatch with record_rows=True')
+    if self._scorer is None:
+      from bsuite_b200 import scoring  # pylint: disable=import-outside-toplevel
+      self._scorer = scoring.Scorer(self.envs)
+    return self._scorer.run(out)
+
   def bytes_per_step(self) -> int:
     """Algorithmic bytes of one lock-step of the whole local batch (SURVEY.md 8d: dense observation + action +
     reward + discount + step_type + compact lane state read and written)."""
     return sum(env.batch * algorithmic_bytes_per_lane_step(env) for env in self.envs.values())
 
   def close(self):
+    if self._scorer is not None:
+      self._scorer.close()
+      self._scorer = None
     for env in self.envs.values():
       env.close()

@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define BSB_ABI_VERSION 6
+#define BSB_ABI_VERSION 7
 #define BSB_DEVICE_HOST (-1)
 #define BSB_MAX_INFO 4
 
@@ -401,6 +401,83 @@ int32_t bsb_comm_world(const bsb_comm* comm, int32_t* rank, int32_t* world);
 int32_t bsb_log_point(bsb_comm* comm, bsb_env* const* envs, int32_t count,
                       double* local, double* gathered, void* stream);
 int32_t bsb_comm_wait(bsb_comm* comm, void* stream);
+
+/*
+ * Scores (experiments/<name>/analysis.py::score, experiments/summary_analysis.py::bsuite_score and
+ * ave_score_by_tag) computed from the per-lane log rows, without the rows leaving the device.
+ *
+ * Every lane is one run of the bsuite: lane j's score for an experiment is what the reference's score(df) returns
+ * for the DataFrame holding lane j's rows of that experiment's ids (with the sweep metadata joined), i.e. what
+ * csv_load.load_bsuite would read back from lane j's CSV files.  Only the ids given to the scorer count.  A lane
+ * with no row of an experiment has that experiment "not scored": score NaN, finished 0.  A tag average is the
+ * NaN-skipping mean over the experiments carrying the tag (NaN when there is none).
+ *
+ * bsb_experiment is the reference's registration order (bsuite/sweep.py); bsb_tag is the tag names sorted.
+ */
+typedef enum bsb_experiment {
+  BSB_EXP_BANDIT = 0, BSB_EXP_BANDIT_NOISE = 1, BSB_EXP_BANDIT_SCALE = 2,
+  BSB_EXP_CARTPOLE = 3, BSB_EXP_CARTPOLE_NOISE = 4, BSB_EXP_CARTPOLE_SCALE = 5, BSB_EXP_CARTPOLE_SWINGUP = 6,
+  BSB_EXP_CATCH = 7, BSB_EXP_CATCH_NOISE = 8, BSB_EXP_CATCH_SCALE = 9,
+  BSB_EXP_DEEP_SEA = 10, BSB_EXP_DEEP_SEA_STOCHASTIC = 11, BSB_EXP_DISCOUNTING_CHAIN = 12,
+  BSB_EXP_MEMORY_LEN = 13, BSB_EXP_MEMORY_SIZE = 14,
+  BSB_EXP_MNIST = 15, BSB_EXP_MNIST_NOISE = 16, BSB_EXP_MNIST_SCALE = 17,
+  BSB_EXP_MOUNTAIN_CAR = 18, BSB_EXP_MOUNTAIN_CAR_NOISE = 19, BSB_EXP_MOUNTAIN_CAR_SCALE = 20,
+  BSB_EXP_UMBRELLA_DISTRACT = 21, BSB_EXP_UMBRELLA_LENGTH = 22,
+  BSB_NUM_EXPERIMENTS = 23
+} bsb_experiment;
+
+typedef enum bsb_tag {
+  BSB_TAG_BASIC = 0, BSB_TAG_CREDIT_ASSIGNMENT = 1, BSB_TAG_EXPLORATION = 2, BSB_TAG_GENERALIZATION = 3,
+  BSB_TAG_MEMORY = 4, BSB_TAG_NOISE = 5, BSB_TAG_SCALE = 6,
+  BSB_NUM_TAGS = 7
+} bsb_tag;
+
+/* "bandit", "bandit_noise", ... / "basic", "credit_assignment", ...; NULL when out of range. */
+const char* bsb_experiment_name(int32_t experiment);
+const char* bsb_tag_name(int32_t tag);
+
+/*
+ * The rows of one bsuite_id, in the layout of bsb_read_log_rows: rows float64 [n_points][n_columns][batch] and
+ * counts int32 [batch], in the memory space of `device`, ascending in episode within a lane.  Column indices name
+ * what the experiment's rule reads: col_episode always; col_value the experiment's regret-like column
+ * (total_regret for bandit / catch / mnist / umbrella, raw_return for cartpole / mountain_car, total_return for
+ * cartpole_swingup / discounting_chain, total_bad_episodes for deep_sea, total_perfect for memory); col_best
+ * best_episode for cartpole and cartpole_swingup (-1 elsewhere).  group_key is the sweep setting the rule groups
+ * by: noise_scale / reward_scale (the _noise / _scale experiments), height_threshold (cartpole_swingup), size
+ * (deep_sea), memory_length / num_bits (memory_len / memory_size), n_distractor / chain_length (umbrella_distract /
+ * umbrella_length); ignored by the other experiments.
+ */
+typedef struct bsb_score_source {
+  int32_t experiment;    /* bsb_experiment */
+  int32_t device;        /* BSB_DEVICE_HOST or CUDA ordinal */
+  int64_t batch;
+  int32_t n_points, n_columns;
+  int32_t col_episode, col_value, col_best;
+  int32_t reserved0;
+  double group_key;
+  const double* rows;
+  const int32_t* counts;
+} bsb_score_source;
+
+/* Fills `out` with the row store of a record-rows environment (created with a log schedule): no copy, the scorer
+ * reads the environment's own rows, so the environment must outlive every scorer built from it.  Fails when the
+ * environment records no rows or its family does not run `experiment`. */
+int32_t bsb_score_source_from_env(const bsb_env* env, int32_t experiment, double group_key, bsb_score_source* out);
+
+/*
+ * A scorer is built once (the inputs are validated and a descriptor table is uploaded) and run many times.
+ * Every source must have `batch` lanes on `device`; at most 128 sources per experiment, n_points <= 4096.
+ * bsb_scorer_run writes scores float64 [BSB_NUM_EXPERIMENTS][batch], finished int32 [BSB_NUM_EXPERIMENTS][batch]
+ * (the reference's _is_finished) and tags float64 [BSB_NUM_TAGS][batch], all in the memory space of `device`.
+ * On CUDA it is ONE kernel launch on `stream`, with no allocation and no synchronisation, so it may be captured
+ * into a CUDA graph; it reads the rows as they are when the launch runs.  On BSB_DEVICE_HOST the same rules run
+ * in a host loop.  Calls on one scorer are not thread-safe.
+ */
+typedef struct bsb_scorer bsb_scorer;
+int32_t bsb_scorer_create(const bsb_score_source* sources, int32_t count, int64_t batch, int32_t device,
+                          bsb_scorer** out);
+int32_t bsb_scorer_run(bsb_scorer* scorer, double* scores, int32_t* finished, double* tags, void* stream);
+int32_t bsb_scorer_destroy(bsb_scorer* scorer);
 
 /* Number of kernels this library has launched in this process (bench evidence). */
 int64_t bsb_launch_count(void);
