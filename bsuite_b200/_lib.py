@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # BSB_LIBRARY points the binding at another build of the SAME library (tools/host_sanitize.sh: ASan/UBSan build)
 LIB_PATH = os.environ.get('BSB_LIBRARY') or os.path.join(_HERE, 'libbsuite_b200.so')
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 DEVICE_HOST = -1
 MAX_INFO = 4
 COMM_ID_BYTES = 128
@@ -27,7 +27,7 @@ FAMILY_NAMES = ('deep_sea', 'catch', 'cartpole', 'cartpole_swingup', 'mountain_c
 WRAP_NONE, WRAP_REWARD_NOISE, WRAP_REWARD_SCALE = range(3)
 # enum bsb_rng_kind
 RNG_PHILOX, RNG_MT19937 = range(2)
-FLAG_TRACK_EPISODES = 1
+FLAG_TRACK_EPISODES, FLAG_SCORE_SUMMARY, FLAG_NO_LOG_ROWS = 1, 2, 4          # bsb_config.flags
 HOST_ORDER_AFTER_STREAM, HOST_PRELAUNCH, HOST_FENCE_CALLER, HOST_NO_WAIT = 1, 2, 4, 8      # bsb_step_host flags
 EPISODE_STAT_FIELDS = ('steps', 'episode', 'total_return', 'episode_len', 'episode_return')
 
@@ -42,7 +42,7 @@ class Config(ctypes.Structure):
       ('chain_length', ctypes.c_int32), ('n_distractor', ctypes.c_int32),
       ('num_actions', ctypes.c_int32), ('max_steps', ctypes.c_int32),
       ('num_data', ctypes.c_int32), ('image_rows', ctypes.c_int32), ('image_cols', ctypes.c_int32),
-      ('reserved0', ctypes.c_int32),
+      ('score_experiment', ctypes.c_int32),
       ('unscaled_move_cost', ctypes.c_double),
       ('height_threshold', ctypes.c_double), ('x_threshold', ctypes.c_double), ('timescale', ctypes.c_double),
       ('max_time', ctypes.c_double), ('init_range', ctypes.c_double),
@@ -65,11 +65,14 @@ class ScoreSource(ctypes.Structure):
   _fields_ = [('experiment', ctypes.c_int32), ('device', ctypes.c_int32), ('batch', ctypes.c_int64),
               ('n_points', ctypes.c_int32), ('n_columns', ctypes.c_int32),
               ('col_episode', ctypes.c_int32), ('col_value', ctypes.c_int32), ('col_best', ctypes.c_int32),
-              ('reserved0', ctypes.c_int32), ('group_key', ctypes.c_double),
+              ('layout', ctypes.c_int32), ('group_key', ctypes.c_double),
               ('rows', ctypes.c_void_p), ('counts', ctypes.c_void_p)]
 
 
 NUM_EXPERIMENTS, NUM_TAGS = 23, 7
+SCORE_ROWS, SCORE_SUMMARY = 0, 1                    # bsb_score_source.layout
+# bsb_read_score_summary: the fields of a score summary, in order
+SUMMARY_FIELDS = ('last_episode', 'last_value', 'prev_episode', 'prev_value', 'best', 'first_solved')
 
 
 EXPORTS = {
@@ -99,6 +102,7 @@ EXPORTS = {
                                                     ctypes.c_void_p]),
     'bsb_log_layout': (ctypes.c_int32, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]),
     'bsb_read_log_rows': (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+    'bsb_read_score_summary': (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     'bsb_state_bytes': (ctypes.c_int32, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64)]),
     'bsb_get_state': (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]),
     'bsb_set_state': (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]),
@@ -120,6 +124,7 @@ EXPORTS = {
     'bsb_tag_name': (ctypes.c_char_p, [ctypes.c_int32]),
     'bsb_score_source_from_env': (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_double,
                                                    ctypes.POINTER(ScoreSource)]),
+    'bsb_score_summarize': (ctypes.c_int32, [ctypes.POINTER(ScoreSource), ctypes.c_void_p, ctypes.c_void_p]),
     'bsb_scorer_create': (ctypes.c_int32, [ctypes.POINTER(ScoreSource), ctypes.c_int32, ctypes.c_int64, ctypes.c_int32,
                                            ctypes.POINTER(ctypes.c_void_p)]),
     'bsb_scorer_run': (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,

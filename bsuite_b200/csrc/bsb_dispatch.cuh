@@ -67,9 +67,9 @@ void host_run(const EnvParams& p, const LaunchArgs& a) {
       const StepOut o = lane_transition<F, R, R>(p, lane, L, rng, wrng, action, a.mode, noise);
       if (track) {
         ep.track(p, lane, o, a.step0 + t, after_last);
-        if (p.log_rows && o.step_type == LAST && log_row_due(p, lane)) {
+        if (p.log_next && o.step_type == LAST && log_row_due(p, lane)) {
           F::store(p, lane, L); ep.store(p, lane);
-          log_row_write(p, lane, a.step0 + t + 1);
+          log_point_record(p, lane, a.step0 + t + 1);
         }
       }
       if (a.reward) a.reward[off] = (float)o.reward;

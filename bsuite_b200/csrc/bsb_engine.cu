@@ -6,6 +6,7 @@
 // families must evaluate the reference's expressions operation by operation.)
 #include <cstdio>
 #include <cstdlib>
+#include <cmath>
 #include <cstring>
 #include <atomic>
 #include <chrono>
@@ -164,6 +165,13 @@ int validate(const bsb_config& c, int64_t batch, int* obs_rows, int* obs_cols, i
     for (int64_t k = 0; k < c.log_schedule_len; ++k)
       if (c.log_schedule[k] < 1 || (k > 0 && c.log_schedule[k] <= c.log_schedule[k - 1]))
         return fail(BSB_INVALID_ARGUMENT, "log_schedule must be positive and strictly ascending");
+  }
+  if ((c.flags & BSB_FLAG_NO_LOG_ROWS) && c.log_schedule_len == 0)
+    return fail(BSB_INVALID_ARGUMENT, "BSB_FLAG_NO_LOG_ROWS needs a log schedule");
+  if (c.flags & BSB_FLAG_SCORE_SUMMARY) {
+    if (c.log_schedule_len == 0) return fail(BSB_INVALID_ARGUMENT, "BSB_FLAG_SCORE_SUMMARY needs a log schedule");
+    int rc = check_score_summary(c);
+    if (rc != BSB_OK) return rc;
   }
   return BSB_OK;
 }
@@ -574,8 +582,16 @@ int32_t bsb_create(const bsb_config* config, int64_t batch, int32_t device, uint
     BSB_TRY(env_alloc_t(e, &sched, (size_t)c.log_schedule_len, false));
     BSB_TRY(env_upload(e, sched, c.log_schedule, (size_t)c.log_schedule_len * sizeof(int64_t)));
     p.log_sched = sched; p.n_log_points = (int32_t)c.log_schedule_len;
-    BSB_TRY(env_alloc_t(e, &p.log_rows, (size_t)c.log_schedule_len * (size_t)(5 + e->names.n) * B, true));
+    if (!(c.flags & BSB_FLAG_NO_LOG_ROWS))
+      BSB_TRY(env_alloc_t(e, &p.log_rows, (size_t)c.log_schedule_len * (size_t)(5 + e->names.n) * B, true));
     BSB_TRY(env_alloc_t(e, &p.log_next, B, true));
+  }
+  if (c.flags & BSB_FLAG_SCORE_SUMMARY) {      // per-lane score summary (bsb_scoring.cuh, fold_row); NaN until a row
+    p.score_exp = c.score_experiment;
+    score_summary_columns(c.score_experiment, e->names, &p.score_col_value, &p.score_col_best);
+    BSB_TRY(env_alloc_t(e, &p.score_sum, (size_t)BSB_SCORE_SUMMARY_FIELDS * B, true));
+    const std::vector<double> nans((size_t)BSB_SCORE_SUMMARY_FIELDS * B, NAN);
+    BSB_TRY(env_upload(e, p.score_sum, nans.data(), nans.size() * sizeof(double)));
   }
   // RNG state
   const bool env_rng = family_uses_env_rng(c);
@@ -797,6 +813,7 @@ int32_t bsb_log_layout(const bsb_env* env, int32_t* n_points, int32_t* n_columns
 
 int32_t bsb_read_log_rows(bsb_env* env, double* rows, int32_t* counts, void* stream) {
   if (!env || !rows || !counts) return fail(BSB_INVALID_ARGUMENT, "null argument");
+  if (env->p.log_next && !env->p.log_rows) return fail(BSB_INVALID_ARGUMENT, "environment keeps no log rows (BSB_FLAG_NO_LOG_ROWS)");
   if (!env->p.log_rows) return fail(BSB_INVALID_ARGUMENT, "environment was created without a log schedule");
   { int frc = drain_host_steps(env); if (frc != BSB_OK) return frc; }
   const size_t B = (size_t)env->p.batch;
@@ -807,6 +824,23 @@ int32_t bsb_read_log_rows(bsb_env* env, double* rows, int32_t* counts, void* str
     BSB_CUDA(cudaMemcpyAsync(counts, env->p.log_next, B * sizeof(int32_t), cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream)));
   } else {
     memcpy(rows, env->p.log_rows, row_bytes);
+    memcpy(counts, env->p.log_next, B * sizeof(int32_t));
+  }
+  return BSB_OK;
+}
+
+int32_t bsb_read_score_summary(bsb_env* env, double* summary, int32_t* counts, void* stream) {
+  if (!env || !summary || !counts) return fail(BSB_INVALID_ARGUMENT, "null argument");
+  if (!env->p.score_sum) return fail(BSB_INVALID_ARGUMENT, "environment was created without BSB_FLAG_SCORE_SUMMARY");
+  { int frc = drain_host_steps(env); if (frc != BSB_OK) return frc; }
+  const size_t B = (size_t)env->p.batch;
+  const size_t bytes = (size_t)BSB_SCORE_SUMMARY_FIELDS * B * sizeof(double);
+  if (env->device >= 0) {
+    DeviceGuard guard(env->device);
+    BSB_CUDA(cudaMemcpyAsync(summary, env->p.score_sum, bytes, cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream)));
+    BSB_CUDA(cudaMemcpyAsync(counts, env->p.log_next, B * sizeof(int32_t), cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream)));
+  } else {
+    memcpy(summary, env->p.score_sum, bytes);
     memcpy(counts, env->p.log_next, B * sizeof(int32_t));
   }
   return BSB_OK;

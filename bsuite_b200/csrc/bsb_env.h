@@ -18,6 +18,12 @@ int fail(int code, const std::string& msg);           // records the thread-loca
 const char* last_error_cstr();
 extern std::atomic<int64_t> g_launches;                // kernels launched by this library
 
+// BSB_FLAG_SCORE_SUMMARY (bsb_scoring.cu): check_score_summary validates a configuration (experiment of the
+// family, log schedule a prefix of the experiment's); score_summary_columns finds the row columns the fold reads
+// (value column, best_episode or -1) among the five Logging columns and the family's info fields.
+int check_score_summary(const bsb_config& c);
+void score_summary_columns(int experiment, const InfoNames& names, int32_t* col_value, int32_t* col_best);
+
 #define BSB_CUDA(expr)                                                                   \
   do {                                                                                   \
     cudaError_t e__ = (expr);                                                            \

@@ -7,6 +7,7 @@
 // emit dense tensors warp-cooperatively.
 #pragma once
 #include "bsb_rng.cuh"
+#include "bsb_scoring.cuh"
 
 namespace bsb {
 
@@ -56,8 +57,12 @@ struct EnvParams {
   // row k of lane i = the wrapper's columns at the LAST timestep that made episode == log_sched[k].
   double* log_rows;          // [n_log_points][5 + n_info][B], or null
   const int64_t* log_sched;  // [n_log_points] ascending episode counts at which the reference writes a row
-  int32_t* log_next;         // [B] rows recorded so far (= index of the next schedule entry)
-  int32_t n_log_points, pad_log;
+  int32_t* log_next;         // [B] rows due so far (= index of the next schedule entry), or null without a schedule
+  int32_t n_log_points, score_exp;
+  // Score summary of experiment score_exp (bsb_scoring.cuh, fold_row), folded from the row columns
+  // score_col_value / score_col_best (-1: none) as each row falls due.
+  double* score_sum;         // [kSummaryFields][B], or null
+  int32_t score_col_value, score_col_best;
   // RNG state: env stream and reward-wrapper stream
   uint64_t* rng_pos;  double* rng_gauss;
   uint64_t* wrng_pos; double* wrng_gauss;
@@ -576,15 +581,28 @@ BSB_HD bool log_row_due(const EnvParams& p, int64_t i) {
   const int32_t k = p.log_next[i];
   return k < p.n_log_points && (int64_t)p.ep[p.batch + i] == p.log_sched[k];
 }
-// Records the row: the five Logging columns and bsuite_info() exactly as the reference's `_log_bsuite_data`
-// (wrappers.py:113-125) reads them right after the LAST timestep.  The lane's state, accumulators and info fields
-// must have been stored to memory (F::store, EpisodeStats::store) before the call.
-BSB_HD void log_row_write(const EnvParams& p, int64_t i, int64_t calls) {
-  const int32_t k = p.log_next[i];
+// Column `col` of the row lane i would record now: the five Logging columns, then bsuite_info().
+BSB_HD double row_column(const EnvParams& p, int64_t i, int col, int64_t calls) {
+  return col < 5 ? episode_stat(p, i, col, calls) : p.info[(int64_t)(col - 5) * p.batch + i];
+}
+// Records row k: the five Logging columns and bsuite_info() exactly as the reference's `_log_bsuite_data`
+// (wrappers.py:113-125) reads them right after the LAST timestep.
+BSB_HD void log_row_write(const EnvParams& p, int64_t i, int32_t k, int64_t calls) {
   const int64_t cols = 5 + p.n_info;
   double* row = p.log_rows + ((int64_t)k * cols) * p.batch + i;
   for (int f = 0; f < 5; ++f) row[(int64_t)f * p.batch] = episode_stat(p, i, f, calls);
   for (int f = 0; f < p.n_info; ++f) row[(int64_t)(5 + f) * p.batch] = p.info[(int64_t)f * p.batch + i];
+}
+// A row has fallen due (log_row_due): store it if there is a row store, fold it into the score summary if there is
+// one, and advance the cursor.  The lane's state, accumulators and info fields must have been stored to memory
+// (F::store, EpisodeStats::store) before the call.
+BSB_HD void log_point_record(const EnvParams& p, int64_t i, int64_t calls) {
+  const int32_t k = p.log_next[i];
+  if (p.log_rows) log_row_write(p, i, k, calls);
+  if (p.score_sum)
+    scoring::fold_row(p.score_sum, i, p.batch, p.score_exp, k, episode_stat(p, i, 1, calls),
+                      row_column(p, i, p.score_col_value, calls),
+                      p.score_col_best >= 0 ? row_column(p, i, p.score_col_best, calls) : NAN);
   p.log_next[i] = k + 1;
 }
 

@@ -868,7 +868,7 @@ __global__ void __launch_bounds__(128, BSB_LAUNCH_MIN_BLOCKS(F)) transition_kern
             if (kTrack) {
               eps[k].track(p, lane, o, step0, after_last);
               eps[k].store(p, lane);
-              if (p.log_rows && o.step_type == LAST && log_row_due(p, lane)) log_row_write(p, lane, step0 + 1);
+              if (p.log_next && o.step_type == LAST && log_row_due(p, lane)) log_point_record(p, lane, step0 + 1);
             }
             if (a.stage.reward) a.stage.reward[lane] = (float)o.reward;
             if (a.stage.reward_f64) a.stage.reward_f64[lane] = o.reward;
@@ -985,9 +985,9 @@ __global__ void __launch_bounds__(128, BSB_LAUNCH_MIN_BLOCKS(F)) transition_kern
         const StepOut o = lane_transition<F, R, R>(p, lane, L, rng, wrng, action, a.mode, kNoise);
         if (kTrack) {
           ep.track(p, lane, o, step0 + t, after_last);
-          if (p.log_rows && o.step_type == LAST && log_row_due(p, lane)) {      // <= 49 times per 10 000 episodes
+          if (p.log_next && o.step_type == LAST && log_row_due(p, lane)) {      // <= 49 times per 10 000 episodes
             F::store(p, lane, L); ep.store(p, lane);
-            log_row_write(p, lane, step0 + t + 1);
+            log_point_record(p, lane, step0 + t + 1);
           }
         }
         if (io.reward) io.reward[off] = (float)o.reward;

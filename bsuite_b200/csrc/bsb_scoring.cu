@@ -56,6 +56,20 @@ const char* value_column(int e) {
   return "total_regret";
 }
 
+// The reference Logging wrapper's schedule (wrappers.py:140-147), as recording.log_schedule computes it: the
+// episode counts in [1, NUM_EPISODES] equal to {1, 1.2, 1.4, 1.7, 2, 2.5, 3, 4, ..., 10} x 10^k.
+std::vector<int64_t> experiment_schedule(int e) {
+  static const double kRatios[] = {1., 1.2, 1.4, 1.7, 2., 2.5, 3., 4., 5., 6., 7., 8., 9., 10.};
+  std::vector<int64_t> out;
+  const int64_t n = (int64_t)exp_info(e).num_episodes;
+  for (int64_t count = 1; count <= n; ++count) {
+    const double scale = pow(10.0, floor(log10((double)count)));
+    for (double r : kRatios)
+      if ((double)count == scale * r) { out.push_back(count); break; }
+  }
+  return out;
+}
+
 __global__ void __launch_bounds__(kLanesPerCta * BSB_NUM_EXPERIMENTS)
 score_kernel(const ScoreDesc* __restrict__ descs, const ScoreExp* __restrict__ exps, int64_t B,
              double* __restrict__ scores, int32_t* __restrict__ finished, double* __restrict__ tags) {
@@ -77,6 +91,32 @@ score_kernel(const ScoreDesc* __restrict__ descs, const ScoreExp* __restrict__ e
 
 }  // namespace
 
+namespace bsb {
+
+int check_score_summary(const bsb_config& c) {
+  const int e = c.score_experiment;
+  if (e < 0 || e >= BSB_NUM_EXPERIMENTS) return fail(BSB_INVALID_ARGUMENT, "unknown score_experiment " + std::to_string(e));
+  if (c.family != experiment_family(e))
+    return fail(BSB_INVALID_ARGUMENT, std::string("the environment's family does not run experiment ") + kExperimentNames[e]);
+  const std::vector<int64_t> sched = experiment_schedule(e);
+  if ((size_t)c.log_schedule_len > sched.size() || !std::equal(c.log_schedule, c.log_schedule + c.log_schedule_len, sched.begin()))
+    return fail(BSB_INVALID_ARGUMENT, std::string("a score summary needs a log schedule that is a prefix of ") +
+                                          kExperimentNames[e] + "'s (episodes up to " + std::to_string(sched.back()) + ")");
+  return BSB_OK;
+}
+
+void score_summary_columns(int e, const InfoNames& names, int32_t* col_value, int32_t* col_best) {
+  const char* want = value_column(e);
+  *col_value = want ? -1 : 2;                              // total_return
+  *col_best = -1;
+  for (int k = 0; k < names.n; ++k) {
+    if (want && strcmp(names.names[k], want) == 0) *col_value = 5 + k;
+    if (rule_needs_best(exp_info(e).rule) && strcmp(names.names[k], "best_episode") == 0) *col_best = 5 + k;
+  }
+}
+
+}  // namespace bsb
+
 struct bsb_scorer {
   int device;
   int64_t batch;
@@ -84,6 +124,39 @@ struct bsb_scorer {
   ScoreExp exps[BSB_NUM_EXPERIMENTS];
   void* table;                         // device copy: descs, then exps
 };
+
+namespace {
+
+// The checks a source passes before it is folded or scored (`at` prefixes the message).
+int check_source(const bsb_score_source& s, const std::string& at) {
+  if (s.experiment < 0 || s.experiment >= BSB_NUM_EXPERIMENTS)
+    return fail(BSB_INVALID_ARGUMENT, at + "unknown experiment " + std::to_string(s.experiment));
+  const ExpInfo info = exp_info(s.experiment);
+  if (s.layout != BSB_SCORE_ROWS && s.layout != BSB_SCORE_SUMMARY)
+    return fail(BSB_INVALID_ARGUMENT, at + "unknown layout " + std::to_string(s.layout));
+  if (s.batch <= 0) return fail(BSB_INVALID_ARGUMENT, at + "batch must be positive");
+  if (!s.rows || !s.counts) return fail(BSB_INVALID_ARGUMENT, at + "null rows or counts");
+  if (s.n_points < 1 || s.n_points > kMaxPoints) return fail(BSB_INVALID_ARGUMENT, at + "n_points must be in [1, 4096]");
+  if (s.layout == BSB_SCORE_SUMMARY) {
+    if (s.n_columns != BSB_SCORE_SUMMARY_FIELDS)
+      return fail(BSB_INVALID_ARGUMENT, at + "a score summary has n_columns = " + std::to_string(BSB_SCORE_SUMMARY_FIELDS) + " fields, not " + std::to_string(s.n_columns));
+  } else {
+    if (s.n_columns < 1) return fail(BSB_INVALID_ARGUMENT, at + "n_columns must be positive");
+    auto has = [&](int32_t c) { return c >= 0 && c < s.n_columns; };
+    if (!has(s.col_episode)) return fail(BSB_INVALID_ARGUMENT, at + "missing column: episode");
+    if (!has(s.col_value)) {
+      const char* name = value_column(s.experiment);
+      return fail(BSB_INVALID_ARGUMENT, at + "missing column: " + (name ? name : "total_return") + " (" + kExperimentNames[s.experiment] + ")");
+    }
+    if (rule_needs_best(info.rule) && !has(s.col_best))
+      return fail(BSB_INVALID_ARGUMENT, at + "missing column: best_episode (" + kExperimentNames[s.experiment] + ")");
+  }
+  if (info.grouped && !(s.group_key == s.group_key))
+    return fail(BSB_INVALID_ARGUMENT, at + "group_key is NaN (" + kExperimentNames[s.experiment] + " groups by it)");
+  return BSB_OK;
+}
+
+}  // namespace
 
 extern "C" {
 
@@ -97,23 +170,57 @@ int32_t bsb_score_source_from_env(const bsb_env* env, int32_t experiment, double
   if (!env || !out) return fail(BSB_INVALID_ARGUMENT, "null argument");
   if (experiment < 0 || experiment >= BSB_NUM_EXPERIMENTS)
     return fail(BSB_INVALID_ARGUMENT, "unknown experiment " + std::to_string(experiment));
-  if (!env->p.log_rows) return fail(BSB_INVALID_ARGUMENT, "environment was created without a log schedule (no rows to score)");
+  if (!env->p.log_next) return fail(BSB_INVALID_ARGUMENT, "environment was created without a log schedule (no rows to score)");
+  if (!env->p.log_rows && !env->p.score_sum)
+    return fail(BSB_INVALID_ARGUMENT, "environment keeps neither log rows nor a score summary (BSB_FLAG_NO_LOG_ROWS without BSB_FLAG_SCORE_SUMMARY)");
   if (env->p.family != experiment_family(experiment))
     return fail(BSB_INVALID_ARGUMENT, std::string("the environment's family does not run experiment ") + kExperimentNames[experiment]);
   bsb_score_source s;
   memset(&s, 0, sizeof(s));
   s.experiment = experiment; s.device = env->device; s.batch = env->p.batch;
-  s.n_points = env->p.n_log_points; s.n_columns = 5 + env->names.n;
-  s.col_episode = 1; s.col_value = -1; s.col_best = -1;
-  const char* want = value_column(experiment);
-  for (int k = 0; k < env->names.n; ++k) {
-    if (want && strcmp(env->names.names[k], want) == 0) s.col_value = 5 + k;
-    if (rule_needs_best(exp_info(experiment).rule) && strcmp(env->names.names[k], "best_episode") == 0) s.col_best = 5 + k;
-  }
-  if (!want) s.col_value = 2;                              // total_return
+  s.n_points = env->p.n_log_points;
   s.group_key = group_key;
-  s.rows = env->p.log_rows; s.counts = env->p.log_next;
+  s.counts = env->p.log_next;
+  if (!env->p.log_rows) {
+    if (env->p.score_exp != experiment)
+      return fail(BSB_INVALID_ARGUMENT, std::string("the environment keeps the score summary of ") + kExperimentNames[env->p.score_exp] +
+                                            ", not of " + kExperimentNames[experiment]);
+    s.layout = BSB_SCORE_SUMMARY; s.n_columns = BSB_SCORE_SUMMARY_FIELDS;
+    s.col_episode = s.col_value = s.col_best = -1;
+    s.rows = env->p.score_sum;
+    *out = s;
+    return BSB_OK;
+  }
+  s.layout = BSB_SCORE_ROWS; s.n_columns = 5 + env->names.n;
+  s.col_episode = 1;
+  score_summary_columns(experiment, env->names, &s.col_value, &s.col_best);
+  s.rows = env->p.log_rows;
   *out = s;
+  return BSB_OK;
+}
+
+int32_t bsb_score_summarize(const bsb_score_source* src, double* summary, int32_t* counts) {
+  if (!src || !summary || !counts) return fail(BSB_INVALID_ARGUMENT, "null argument");
+  const bsb_score_source& s = *src;
+  if (s.layout != BSB_SCORE_ROWS) return fail(BSB_INVALID_ARGUMENT, "bsb_score_summarize folds a BSB_SCORE_ROWS source");
+  if (s.device != BSB_DEVICE_HOST) return fail(BSB_INVALID_ARGUMENT, "bsb_score_summarize reads host rows (device BSB_DEVICE_HOST)");
+  { int rc = check_source(s, ""); if (rc != BSB_OK) return rc; }
+  const std::vector<int64_t> sched = experiment_schedule(s.experiment);
+  const int64_t B = s.batch;
+  const bool best = rule_needs_best(exp_info(s.experiment).rule);
+  for (int64_t i = 0; i < (int64_t)BSB_SCORE_SUMMARY_FIELDS * B; ++i) summary[i] = NAN;
+  for (int64_t lane = 0; lane < B; ++lane) {
+    const int32_t c = s.counts[lane] < 0 ? 0 : (s.counts[lane] > s.n_points ? s.n_points : s.counts[lane]);
+    auto at = [&](int32_t k, int32_t col) { return s.rows[((int64_t)k * s.n_columns + col) * B + lane]; };
+    for (int32_t k = 0; k < c; ++k)
+      if ((size_t)k >= sched.size() || at(k, s.col_episode) != (double)sched[(size_t)k])
+        return fail(BSB_INVALID_ARGUMENT, "lane " + std::to_string(lane) + ": row " + std::to_string(k) +
+                                              " is not at episode " + ((size_t)k < sched.size() ? std::to_string(sched[(size_t)k]) : std::string("<none>")) +
+                                              " of " + kExperimentNames[s.experiment] + "'s log schedule (the rows must be a prefix of it)");
+    for (int32_t k = 0; k < c; ++k)
+      fold_row(summary, lane, B, s.experiment, k, at(k, s.col_episode), at(k, s.col_value), best ? at(k, s.col_best) : NAN);
+    counts[lane] = c;
+  }
   return BSB_OK;
 }
 
@@ -128,24 +235,10 @@ int32_t bsb_scorer_create(const bsb_score_source* sources, int32_t count, int64_
   for (int32_t i = 0; i < count; ++i) {
     const bsb_score_source& s = sources[i];
     const std::string at = "source " + std::to_string(i) + ": ";
-    if (s.experiment < 0 || s.experiment >= BSB_NUM_EXPERIMENTS)
-      return fail(BSB_INVALID_ARGUMENT, at + "unknown experiment " + std::to_string(s.experiment));
-    const ExpInfo info = exp_info(s.experiment);
+    int rc = check_source(s, at);
+    if (rc != BSB_OK) return rc;
     if (s.batch != batch) return fail(BSB_INVALID_ARGUMENT, at + "batch " + std::to_string(s.batch) + " differs from the scorer's " + std::to_string(batch));
     if (s.device != device) return fail(BSB_INVALID_ARGUMENT, at + "lives on another device than the scorer");
-    if (!s.rows || !s.counts) return fail(BSB_INVALID_ARGUMENT, at + "null rows or counts");
-    if (s.n_points < 1 || s.n_points > kMaxPoints) return fail(BSB_INVALID_ARGUMENT, at + "n_points must be in [1, 4096]");
-    if (s.n_columns < 1) return fail(BSB_INVALID_ARGUMENT, at + "n_columns must be positive");
-    auto has = [&](int32_t c) { return c >= 0 && c < s.n_columns; };
-    if (!has(s.col_episode)) return fail(BSB_INVALID_ARGUMENT, at + "missing column: episode");
-    if (!has(s.col_value)) {
-      const char* name = value_column(s.experiment);
-      return fail(BSB_INVALID_ARGUMENT, at + "missing column: " + (name ? name : "total_return") + " (" + kExperimentNames[s.experiment] + ")");
-    }
-    if (rule_needs_best(info.rule) && !has(s.col_best))
-      return fail(BSB_INVALID_ARGUMENT, at + "missing column: best_episode (" + kExperimentNames[s.experiment] + ")");
-    if (info.grouped && !(s.group_key == s.group_key))
-      return fail(BSB_INVALID_ARGUMENT, at + "group_key is NaN (" + kExperimentNames[s.experiment] + " groups by it)");
     if (++per_exp[s.experiment] > kMaxSourcesPerExperiment)
       return fail(BSB_INVALID_ARGUMENT, std::string("more than 128 sources for experiment ") + kExperimentNames[s.experiment]);
   }
@@ -165,15 +258,17 @@ int32_t bsb_scorer_create(const bsb_score_source* sources, int32_t count, int64_
   });
   bsb_scorer* sc = new bsb_scorer();
   sc->device = device; sc->batch = batch; sc->table = nullptr;
-  for (int e = 0; e < BSB_NUM_EXPERIMENTS; ++e) sc->exps[e] = ScoreExp{0, 0};
+  for (int e = 0; e < BSB_NUM_EXPERIMENTS; ++e) sc->exps[e] = ScoreExp{0, 0, kViewRows, 0};
   for (int32_t i : order) {
     const bsb_score_source& s = sources[i];
     ScoreDesc d;
     d.rows = s.rows; d.counts = s.counts; d.n_points = s.n_points; d.n_columns = s.n_columns;
-    d.col_episode = s.col_episode; d.col_value = s.col_value; d.col_best = s.col_best; d.reserved0 = 0;
+    d.col_episode = s.col_episode; d.col_value = s.col_value; d.col_best = s.col_best; d.layout = s.layout;
     d.key = s.group_key;
     ScoreExp& ex = sc->exps[s.experiment];
-    if (ex.count == 0) ex.first = (int32_t)sc->descs.size();
+    const int32_t view = s.layout == BSB_SCORE_SUMMARY ? kViewSummary : kViewRows;
+    if (ex.count == 0) { ex.first = (int32_t)sc->descs.size(); ex.view = view; }
+    else if (ex.view != view) ex.view = kViewMixed;
     ++ex.count;
     sc->descs.push_back(d);
   }

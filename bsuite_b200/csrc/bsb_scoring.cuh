@@ -25,16 +25,18 @@ namespace scoring {
 constexpr int kMaxSourcesPerExperiment = 128;   // NpSum restates numpy's pairwise sum for n <= 128 terms
 constexpr int kMaxPoints = 4096;
 
-// One bsuite_id's rows (bsb_score_source, as uploaded).  Within an experiment the descriptors of a grouping rule
-// are sorted by group key (stable), so a group is a contiguous run.
+// One bsuite_id's rows or score summary (bsb_score_source, as uploaded).  Within an experiment the descriptors of a
+// grouping rule are sorted by group key (stable), so a group is a contiguous run.
 struct ScoreDesc {
-  const double* rows;      // [n_points][n_columns][B]
+  const double* rows;      // [n_points][n_columns][B] (BSB_SCORE_ROWS) or [kSummaryFields][B] (BSB_SCORE_SUMMARY)
   const int32_t* counts;   // [B]
-  int32_t n_points, n_columns, col_episode, col_value, col_best, reserved0;
+  int32_t n_points, n_columns, col_episode, col_value, col_best, layout;
   double key;
 };
 
-struct ScoreExp { int32_t first, count; };     // descriptor range of one experiment
+// Descriptor range of one experiment, and the layouts among them: kViewRows, kViewSummary or kViewMixed.
+struct ScoreExp { int32_t first, count, view, pad; };
+enum View : int32_t { kViewRows, kViewSummary, kViewMixed };
 
 enum Rule : int32_t {
   kRegret,          // bandit, catch (+ _noise / _scale): ave_regret_score on total_regret
@@ -93,6 +95,33 @@ BSB_SC_HD bool rule_needs_best(int rule) { return rule == kCartpole || rule == k
 // cartpole, cartpole_swingup and deep_sea keep only episode <= NUM_EPISODES (their preprocessors / find_solution)
 BSB_SC_HD bool rule_caps_episodes(int rule) { return rule == kCartpole || rule == kSwingup || rule == kDeepSea; }
 
+// Score summary of one id and lane (bsb_read_score_summary), field f at summary[f * B + lane].
+enum SummaryField { kLastEpisode, kLastValue, kPrevEpisode, kPrevValue, kBest, kFirstSolved, kSummaryFields };
+static_assert(kSummaryFields == BSB_SCORE_SUMMARY_FIELDS, "summary layout");
+
+// Folds row k (k rows came before it) of one lane into its summary.  The rows of an id are a prefix of the log
+// schedule, so the rules need only what is folded here (Lane<SummaryView> below): the latest row (the row at
+// n_eps of mean_regret_at_last, _is_finished, the last episode of deep_sea), the row before it (mnist's diff()
+// term: 10 000 is the only schedule point past 0.9 NUM_EPISODES), the running max of best_episode in the scan's
+// own comparison order (solved_fraction), and deep_sea's first solved episode among the rows range() keeps.
+// episode, value and best are the row's columns col_episode, col_value and col_best, the doubles the row store
+// holds; `best` is not read where the rule has no best_episode.
+BSB_SC_HD void fold_row(double* summary, int64_t lane, int64_t B, int experiment, int32_t k, double episode,
+                        double value, double best) {
+  const ExpInfo info = exp_info(experiment);
+  double* s = summary + lane;
+  if (k == 0) {
+    s[kPrevEpisode * B] = NAN; s[kPrevValue * B] = NAN; s[kBest * B] = NAN; s[kFirstSolved * B] = NAN;
+  } else {
+    s[kPrevEpisode * B] = s[kLastEpisode * B]; s[kPrevValue * B] = s[kLastValue * B];
+  }
+  s[kLastEpisode * B] = episode; s[kLastValue * B] = value;
+  if (rule_needs_best(info.rule) && (k == 0 || best > s[kBest * B])) s[kBest * B] = best;
+  if (info.rule == kDeepSea && !(s[kFirstSolved * B] == s[kFirstSolved * B]) &&
+      !(episode < (double)info.min_episode) && !(episode > info.num_episodes) && value / episode < info.base)
+    s[kFirstSolved * B] = episode;
+}
+
 // numpy's pairwise summation (the order of np.sum / np.mean and of pandas' Series.mean) for n <= 128 terms, fed
 // one term at a time: below 8 terms a running sum; otherwise 8 interleaved partial sums, combined as
 // ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)), then the n % 8 trailing terms one by one.
@@ -116,8 +145,10 @@ struct NpSum {
 
 BSB_SC_HD double clip01(double x) { return x < 0.0 ? 0.0 : (x > 1.0 ? 1.0 : x); }   // np.clip keeps NaN
 
-// One lane of one experiment.
-struct Lane {
+// What the rules read of one id's rows, over the row store (RowView: the scans) or a score summary (SummaryView:
+// the folded fields).  Row indices are those of the row store; a summary holds the last two rows of an id only,
+// which is every row the rules index (see fold_row), and reads NaN elsewhere.
+struct RowView {
   const ScoreDesc* d;      // the experiment's descriptors
   int64_t lane, B;
   ExpInfo info;
@@ -146,6 +177,94 @@ struct Lane {
     while (k >= lo && ep(s, k) > e) --k;
     return (k >= lo && ep(s, k) == e) ? k : -1;
   }
+  // max of best_episode over rows [lo, hi) (hi > lo), in the order of np.max's scan.
+  BSB_SC_HD double best(int s, int lo, int hi) const {
+    double best = at(s, lo, d[s].col_best);
+    for (int k = lo + 1; k < hi; ++k) { const double b = at(s, k, d[s].col_best); if (b > best) best = b; }
+    return best;
+  }
+  // Episode of the first row in [lo, hi) with value / episode < threshold (deep_sea's find_solution).
+  BSB_SC_HD bool first_solved(int s, int lo, int hi, double* first) const {
+    for (int k = lo; k < hi; ++k) {
+      const double e = ep(s, k);
+      if (value(s, k) / e < info.base) { *first = e; return true; }
+    }
+    return false;
+  }
+};
+
+struct SummaryView {
+  const ScoreDesc* d;
+  int64_t lane, B;
+  ExpInfo info;
+
+  BSB_SC_HD double field(int s, int f) const { return d[s].rows[(int64_t)f * B + lane]; }
+  BSB_SC_HD double ep(int s, int k) const {
+    const int c = count(s);
+    return k == c - 1 ? field(s, kLastEpisode) : (k == c - 2 ? field(s, kPrevEpisode) : NAN);
+  }
+  BSB_SC_HD double value(int s, int k) const {
+    const int c = count(s);
+    return k == c - 1 ? field(s, kLastValue) : (k == c - 2 ? field(s, kPrevValue) : NAN);
+  }
+  BSB_SC_HD int count(int s) const {
+    int c = d[s].counts[lane];
+    return c < 0 ? 0 : (c > d[s].n_points ? d[s].n_points : c);
+  }
+  // Every row of a schedule prefix is <= NUM_EPISODES (no cap), and the rows below min_episode are a prefix of
+  // them: the rule keeps rows iff the last one is kept.  lo is only handed back to the queries below.
+  BSB_SC_HD void range(int s, int* lo, int* hi) const {
+    const int h = count(s);
+    *hi = h;
+    *lo = (h > 0 && info.min_episode > 0 && field(s, kLastEpisode) < (double)info.min_episode) ? h : 0;
+  }
+  // e is a schedule point whenever the rules ask (an id's last episode, or a first solved one), so the kept rows
+  // hold it iff min_episode <= e <= last.  Only the last row is ever read back; an earlier one is reported as lo.
+  BSB_SC_HD int row_at_episode(int s, int lo, int hi, double e) const {
+    if (hi <= lo) return -1;
+    const double last = field(s, kLastEpisode);
+    if (e == last) return hi - 1;
+    return (e < last && !(e < (double)info.min_episode)) ? lo : -1;
+  }
+  BSB_SC_HD double best(int s, int, int) const { return field(s, kBest); }
+  BSB_SC_HD bool first_solved(int s, int, int, double* first) const {
+    const double f = field(s, kFirstSolved);
+    if (!(f == f)) return false;
+    *first = f;
+    return true;
+  }
+};
+
+// Sources of both layouts within one experiment: each id is read through its own descriptor's view.
+struct MixedView {
+  RowView r;
+  SummaryView m;
+  BSB_SC_HD bool sm(int s) const { return r.d[s].layout == BSB_SCORE_SUMMARY; }
+  BSB_SC_HD double ep(int s, int k) const { return sm(s) ? m.ep(s, k) : r.ep(s, k); }
+  BSB_SC_HD double value(int s, int k) const { return sm(s) ? m.value(s, k) : r.value(s, k); }
+  BSB_SC_HD int count(int s) const { return sm(s) ? m.count(s) : r.count(s); }
+  BSB_SC_HD void range(int s, int* lo, int* hi) const { if (sm(s)) m.range(s, lo, hi); else r.range(s, lo, hi); }
+  BSB_SC_HD int row_at_episode(int s, int lo, int hi, double e) const {
+    return sm(s) ? m.row_at_episode(s, lo, hi, e) : r.row_at_episode(s, lo, hi, e);
+  }
+  BSB_SC_HD double best(int s, int lo, int hi) const { return sm(s) ? m.best(s, lo, hi) : r.best(s, lo, hi); }
+  BSB_SC_HD bool first_solved(int s, int lo, int hi, double* first) const {
+    return sm(s) ? m.first_solved(s, lo, hi, first) : r.first_solved(s, lo, hi, first);
+  }
+};
+
+// One lane of one experiment, read through view V.
+template <class V>
+struct Lane {
+  V v;
+  const ScoreDesc* d;      // the experiment's descriptors
+  ExpInfo info;
+
+  BSB_SC_HD double ep(int s, int k) const { return v.ep(s, k); }
+  BSB_SC_HD double value(int s, int k) const { return v.value(s, k); }
+  BSB_SC_HD int count(int s) const { return v.count(s); }
+  BSB_SC_HD void range(int s, int* lo, int* hi) const { v.range(s, lo, hi); }
+  BSB_SC_HD int row_at_episode(int s, int lo, int hi, double e) const { return v.row_at_episode(s, lo, hi, e); }
   // The column ave_regret_score averages, as the preprocessors derive it.
   BSB_SC_HD double regret(int s, int k) const {
     const double e = ep(s, k), v = value(s, k);
@@ -192,8 +311,7 @@ struct Lane {
     for (int s = s0; s < s1; ++s) {
       int lo, hi; range(s, &lo, &hi);
       if (hi <= lo) continue;
-      double best = at(s, lo, d[s].col_best);
-      for (int k = lo + 1; k < hi; ++k) { const double b = at(s, k, d[s].col_best); if (b > best) best = b; }
+      const double best = v.best(s, lo, hi);
       ++ids; hits += best > good;
     }
     return (double)hits / (double)ids;
@@ -302,13 +420,10 @@ struct Lane {
         const double e_last = ep(u, hi - 1);
         if (!any || e_last > last) last = e_last;
         any = true;
-        for (int k = lo; k < hi; ++k) {
-          const double e = ep(u, k);
-          if (value(u, k) / e < info.base) {
-            if (!solved || e < first) first = e;
-            solved = true;
-            break;
-          }
+        double e;
+        if (v.first_solved(u, lo, hi, &e)) {
+          if (!solved || e < first) first = e;
+          solved = true;
         }
       }
       if (!any) continue;
@@ -331,11 +446,9 @@ struct Lane {
 
 struct ScoreOut { double score; int32_t finished; int32_t present; };
 
-BSB_SC_HD ScoreOut score_lane(const ScoreDesc* descs, ScoreExp ex, int e, int64_t lane, int64_t B) {
+template <class V>
+BSB_SC_HD ScoreOut score_lane_as(const Lane<V>& L, int n) {
   ScoreOut out = {NAN, 0, 0};
-  if (ex.count <= 0) return out;
-  Lane L{descs + ex.first, lane, B, exp_info(e)};
-  const int n = ex.count;
   // _is_finished: every id with rows has reached NUM_EPISODES (on the unfiltered rows)
   double min_last = 0.0;
   bool any = false;
@@ -359,6 +472,19 @@ BSB_SC_HD ScoreOut score_lane(const ScoreDesc* descs, ScoreExp ex, int e, int64_
     default: out.score = L.base_score(0, n); break;
   }
   return out;
+}
+
+BSB_SC_HD ScoreOut score_lane(const ScoreDesc* descs, ScoreExp ex, int e, int64_t lane, int64_t B) {
+  if (ex.count <= 0) return ScoreOut{NAN, 0, 0};
+  const ScoreDesc* d = descs + ex.first;
+  const ExpInfo info = exp_info(e);
+  const RowView rows{d, lane, B, info};
+  const SummaryView summary{d, lane, B, info};
+  switch (ex.view) {
+    case kViewSummary: return score_lane_as(Lane<SummaryView>{summary, d, info}, ex.count);
+    case kViewMixed: return score_lane_as(Lane<MixedView>{MixedView{rows, summary}, d, info}, ex.count);
+  }
+  return score_lane_as(Lane<RowView>{rows, d, info}, ex.count);
 }
 
 // ave_score_by_tag for one lane: pandas' NaN-skipping mean over the scored experiments carrying the tag (NaN

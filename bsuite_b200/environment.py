@@ -50,12 +50,13 @@ def _resolve_device(device) -> int:
   return dev.index if dev.index is not None else torch.cuda.current_device()
 
 
-def _make_config(spec: EnvSpec, rng_kind: int, flags: int, log_schedule=None):
+def _make_config(spec: EnvSpec, rng_kind: int, flags: int, log_schedule=None, score_experiment: int = 0):
   cfg = _lib.Config()
   cfg.family = spec.family
   cfg.wrapper = spec.wrapper
   cfg.rng_kind = rng_kind
   cfg.flags = flags
+  cfg.score_experiment = score_experiment
   cfg.deterministic = 1
   cfg.reward_scale = 1.0
   for key, value in spec.fields.items():
@@ -83,9 +84,9 @@ class _Handle:
   """Owns one bsb_env*."""
 
   def __init__(self, spec: EnvSpec, batch: int, device_ordinal: int, seed: int, lane_offset: int,
-               rng_kind: int, flags: int, log_schedule=None):
+               rng_kind: int, flags: int, log_schedule=None, score_experiment: int = 0):
     self.lib = _lib.load()
-    cfg, keep = _make_config(spec, rng_kind, flags, log_schedule)
+    cfg, keep = _make_config(spec, rng_kind, flags, log_schedule, score_experiment)
     ptr = ctypes.c_void_p()
     _lib.check(self.lib.bsb_create(ctypes.byref(cfg), batch, device_ordinal, seed & _MASK64,
                                    lane_offset & _MASK64, ctypes.byref(ptr)))
@@ -168,7 +169,8 @@ class BatchedEnvironment:
 
   def __init__(self, spec: EnvSpec, batch: int, device='cuda', seed: Optional[int] = None,
                rng: str = 'philox', lane_offset: int = 0, track_episodes: bool = False,
-               reward_dtype='float32', record_rows: bool = False):
+               reward_dtype='float32', record_rows: bool = False, track_scores: bool = False,
+               score_experiment: Optional[str] = None):
     import torch
     self._torch = torch
     self._spec = spec
@@ -188,16 +190,29 @@ class BatchedEnvironment:
     self._async_work = False        # something was enqueued on a torch stream since the last host-driven step
     # record_rows: every lane keeps the rows the reference's Logging wrapper would have written for it, at the
     # log-spaced episode counts of utils/wrappers.py:140-147 (recording.write_lane_csvs turns them into files)
-    track_episodes = bool(track_episodes or record_rows)
+    # track_scores: every lane keeps only what experiment `score_experiment`'s scoring rule reads of those rows (a
+    # score summary, 48 bytes per lane), folded in as the rows fall due; scoring.Scorer scores from it
+    track_episodes = bool(track_episodes or record_rows or track_scores)
     flags = _lib.FLAG_TRACK_EPISODES if track_episodes else 0
     self._track = bool(track_episodes)
+    self._record_rows, self._track_scores = bool(record_rows), bool(track_scores)
     self._log_schedule = None
-    if record_rows:
+    self._score_experiment = None
+    experiment_index = 0
+    if record_rows or track_scores:
       from bsuite_b200 import recording  # pylint: disable=import-outside-toplevel
       self._log_schedule = recording.log_schedule(spec.bsuite_num_episodes)
+    if track_scores:
+      from bsuite_b200 import scoring  # pylint: disable=import-outside-toplevel
+      if score_experiment not in scoring.EXPERIMENTS:
+        raise ValueError(f'track_scores=True needs score_experiment, one of the 23 experiment names (got '
+                         f'{score_experiment!r}); load / load_from_id set it')
+      self._score_experiment = score_experiment
+      experiment_index = scoring.EXPERIMENTS.index(score_experiment)
+      flags |= _lib.FLAG_SCORE_SUMMARY | (0 if record_rows else _lib.FLAG_NO_LOG_ROWS)
     self._reward_dtype = torch.float64 if str(reward_dtype).endswith('64') else torch.float32
     self._handle = _Handle(spec, self._batch, self._ordinal, self._seed, self._lane_offset, self._rng_kind, flags,
-                           self._log_schedule)
+                           self._log_schedule, experiment_index)
     self._lib = self._handle.lib
     n = ctypes.c_int32()
     _lib.check(self._lib.bsb_info_count(self._handle.ptr, ctypes.byref(n)))
@@ -481,7 +496,7 @@ class BatchedEnvironment:
     """The per-lane log rows recorded on the device (`record_rows=True`): `columns` (the reference wrapper's five
     columns + the bsuite_info() keys), `rows` float64 [n_points, n_columns, B], `counts` int32 [B] (rows recorded
     so far per lane) and `schedule` (episode count of every row index)."""
-    if self._log_schedule is None:
+    if not self._record_rows:
       raise RuntimeError('create the environment with record_rows=True')
     torch = self._torch
     n_points, n_cols = ctypes.c_int32(), ctypes.c_int32()
@@ -491,6 +506,20 @@ class BatchedEnvironment:
     _lib.check(self._lib.bsb_read_log_rows(self._handle.ptr, rows.data_ptr(), counts.data_ptr(), self._stream()))
     return dict(columns=_lib.EPISODE_STAT_FIELDS + self._info_names, rows=rows, counts=counts,
                 schedule=np.asarray(self._log_schedule))
+
+  def score_summary(self) -> Dict[str, Any]:
+    """The per-lane score summary kept on the device (`track_scores=True`): float64 [B] per field of
+    `_lib.SUMMARY_FIELDS` (bsb_read_score_summary explains them), `counts` int32 [B] (rows folded in so far per
+    lane), `n_points` (length of the log schedule) and `experiment` (the experiment it is kept for)."""
+    if not self._track_scores:
+      raise RuntimeError('create the environment with track_scores=True')
+    torch = self._torch
+    block = torch.empty((len(_lib.SUMMARY_FIELDS), self._batch), dtype=torch.float64, device=self._device)
+    counts = torch.empty(self._batch, dtype=torch.int32, device=self._device)
+    _lib.check(self._lib.bsb_read_score_summary(self._handle.ptr, block.data_ptr(), counts.data_ptr(), self._stream()))
+    result = {name: block[f] for f, name in enumerate(_lib.SUMMARY_FIELDS)}
+    result.update(counts=counts, n_points=len(self._log_schedule), experiment=self._score_experiment)
+    return result
 
   def episode_stat_sums(self, out=None):
     """Sums over this environment's lanes of (steps, episode, total_return, episode_len, episode_return): a float64
@@ -530,8 +559,11 @@ class BatchedEnvironment:
     """Everything that shapes the meaning of the snapshot bytes besides (batch, family, seed, lane_offset)."""
     import hashlib
     h = hashlib.sha256()
-    h.update(repr((sorted(self._spec.fields.items()), self._spec.wrapper, self._rng_kind, self._track,
-                   tuple(self._spec.obs_shape), self._spec.num_actions)).encode())
+    key = (sorted(self._spec.fields.items()), self._spec.wrapper, self._rng_kind, self._track,
+           tuple(self._spec.obs_shape), self._spec.num_actions)
+    if self._track_scores:                # only when on: the fingerprints of other configurations stay as they were
+      key += (('track_scores', self._score_experiment, self._record_rows),)
+    h.update(repr(key).encode())
     for table in (self._spec.table, self._spec.table2):
       if table is not None:
         h.update(np.ascontiguousarray(table).tobytes())

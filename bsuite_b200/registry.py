@@ -33,6 +33,8 @@ def load(experiment_name: str, kwargs: Mapping[str, Any], batch: Optional[int] =
          seed: Optional[int] = None, rng: Optional[str] = None, **engine_kwargs):
   """Returns a bsuite environment given an experiment name and settings (bsuite.py:93-98)."""
   spec = experiments.EXPERIMENT_NAME_TO_SPEC[experiment_name](**kwargs)
+  if engine_kwargs.get('track_scores'):      # the score summary is the experiment's
+    engine_kwargs.setdefault('score_experiment', experiment_name)
   return _instantiate(spec, batch, device, seed, rng, **engine_kwargs)
 
 

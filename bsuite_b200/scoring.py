@@ -12,6 +12,11 @@ in one kernel launch for a whole sweep (`bsb_scorer_run`), without writing or re
 
 Row i of `scores` / `finished` is experiment `EXPERIMENTS[i]`, row t of `tags` is tag `TAGS[t]`.  An experiment
 without a row in a lane is not scored there (NaN, finished 0); a tag average skips NaN, as pandas' mean does.
+
+Scores need far less than the rows: `track_scores=True` instead of `record_rows=True` keeps, per id and lane, a
+score summary of six float64 values (`_lib.SUMMARY_FIELDS`), folded in on the device as each row falls due.  A
+lane's rows are always a prefix of the log schedule, so the summary holds everything the scoring rules read of
+them, and the scores from summaries are the same bits as the scores from the rows.
 """
 
 import ctypes
@@ -72,11 +77,13 @@ class Scorer:
   """
 
   def __init__(self, envs_by_id: Mapping[str, Any]):
+    """Reads an environment's rows when it records them (`record_rows=True`), its score summary otherwise
+    (`track_scores=True`); both give the same scores."""
     sources = []
     lib = _lib.load()
     for bsuite_id, env in envs_by_id.items():
-      if getattr(env, '_log_schedule', None) is None:
-        raise ValueError(f'{bsuite_id}: create the environment with record_rows=True to score it')
+      if not (getattr(env, '_record_rows', False) or getattr(env, '_track_scores', False)):
+        raise ValueError(f'{bsuite_id}: create the environment with record_rows=True or track_scores=True to score it')
       experiment = EXPERIMENTS.index(experiment_of(bsuite_id))
       source = _lib.ScoreSource()
       _lib.check(lib.bsb_score_source_from_env(env._handle.ptr, experiment, group_key(bsuite_id),  # pylint: disable=protected-access
@@ -88,31 +95,51 @@ class Scorer:
     self._init(sources, first.batch, first.device, keep=dict(envs_by_id))
 
   @classmethod
-  def from_rows(cls, tables: Mapping[str, Mapping[str, Any]], device='cpu') -> 'Scorer':
+  def from_rows(cls, tables: Mapping[str, Mapping[str, Any]], device='cpu', summarize: bool = False) -> 'Scorer':
     """A scorer over caller-owned rows: bsuite_id -> dict(rows=[n_points, n_columns, B] float64,
     counts=[B] int32, columns=names of the n_columns columns), numpy arrays or tensors (copied to `device` when
-    they are not already there as contiguous tensors of those dtypes)."""
+    they are not already there as contiguous tensors of those dtypes).  summarize=True folds the rows into score
+    summaries on the host first (`summarize`) and scores those on `device`."""
     import torch
     device = torch.device(device)
+    if summarize:
+      return cls.from_summaries({bsuite_id: _summarize(bsuite_id, table)
+                                 for bsuite_id, table in tables.items()}, device=device)
     sources, keep, batch = [], [], None
     for bsuite_id, table in tables.items():
-      name = experiment_of(bsuite_id)
-      rows = torch.as_tensor(table['rows']).to(device=device, dtype=torch.float64).contiguous()
-      counts = torch.as_tensor(table['counts']).to(device=device, dtype=torch.int32).contiguous()
-      columns = list(table['columns'])
-      if rows.dim() != 3 or rows.shape[1] != len(columns) or counts.shape != (rows.shape[2],):
-        raise ValueError(f'{bsuite_id}: rows must be [n_points, len(columns), B] and counts [B]')
-      index = lambda c: columns.index(c) if c in columns else -1
-      source = _lib.ScoreSource(
-          experiment=EXPERIMENTS.index(name), device=_lib.DEVICE_HOST if device.type == 'cpu' else device.index or 0,
-          batch=rows.shape[2], n_points=rows.shape[0], n_columns=rows.shape[1], col_episode=index('episode'),
-          col_value=index(VALUE_COLUMNS[name]), col_best=index('best_episode') if name in NEEDS_BEST else -1,
-          group_key=group_key(bsuite_id), rows=rows.data_ptr(), counts=counts.data_ptr())
+      source, rows, counts = _rows_source(bsuite_id, table, device)
       sources.append(source)
       keep += [rows, counts]
       batch = rows.shape[2] if batch is None else batch
     if not sources:
       raise ValueError('no rows to score')
+    scorer = cls.__new__(cls)
+    scorer._init(sources, batch, device, keep=keep)  # pylint: disable=protected-access
+    return scorer
+
+  @classmethod
+  def from_summaries(cls, summaries: Mapping[str, Mapping[str, Any]], device='cpu') -> 'Scorer':
+    """A scorer over caller-owned score summaries: bsuite_id -> dict as `summarize` or
+    `BatchedEnvironment.score_summary` return it (a float64 [B] per field of `_lib.SUMMARY_FIELDS`, counts [B],
+    n_points), copied to `device`."""
+    import torch
+    device = torch.device(device)
+    sources, keep, batch = [], [], None
+    for bsuite_id, summary in summaries.items():
+      block = torch.stack([torch.as_tensor(summary[f]).to(device=device, dtype=torch.float64)
+                           for f in _lib.SUMMARY_FIELDS]).contiguous()
+      counts = torch.as_tensor(summary['counts']).to(device=device, dtype=torch.int32).contiguous()
+      if block.dim() != 2 or counts.shape != (block.shape[1],):
+        raise ValueError(f'{bsuite_id}: every summary field and counts must be [B]')
+      sources.append(_lib.ScoreSource(
+          experiment=EXPERIMENTS.index(experiment_of(bsuite_id)), device=_ordinal(device), batch=block.shape[1],
+          n_points=int(summary['n_points']), n_columns=block.shape[0], col_episode=-1, col_value=-1, col_best=-1,
+          layout=_lib.SCORE_SUMMARY, group_key=group_key(bsuite_id), rows=block.data_ptr(),
+          counts=counts.data_ptr()))
+      keep += [block, counts]
+      batch = block.shape[1] if batch is None else batch
+    if not sources:
+      raise ValueError('no summaries to score')
     scorer = cls.__new__(cls)
     scorer._init(sources, batch, device, keep=keep)  # pylint: disable=protected-access
     return scorer
@@ -169,6 +196,49 @@ class Scorer:
       self.close()
     except Exception:  # pylint: disable=broad-except
       pass
+
+
+def _ordinal(device) -> int:
+  return _lib.DEVICE_HOST if device.type == 'cpu' else (device.index or 0)
+
+
+def _rows_source(bsuite_id: str, table: Mapping[str, Any], device):
+  """A BSB_SCORE_ROWS source over `table` (see Scorer.from_rows), and the tensors it points at."""
+  import torch
+  name = experiment_of(bsuite_id)
+  rows = torch.as_tensor(table['rows']).to(device=device, dtype=torch.float64).contiguous()
+  counts = torch.as_tensor(table['counts']).to(device=device, dtype=torch.int32).contiguous()
+  columns = list(table['columns'])
+  if rows.dim() != 3 or rows.shape[1] != len(columns) or counts.shape != (rows.shape[2],):
+    raise ValueError(f'{bsuite_id}: rows must be [n_points, len(columns), B] and counts [B]')
+  index = lambda c: columns.index(c) if c in columns else -1
+  source = _lib.ScoreSource(
+      experiment=EXPERIMENTS.index(name), device=_ordinal(device),
+      batch=rows.shape[2], n_points=rows.shape[0], n_columns=rows.shape[1], col_episode=index('episode'),
+      col_value=index(VALUE_COLUMNS[name]), col_best=index('best_episode') if name in NEEDS_BEST else -1,
+      group_key=group_key(bsuite_id), rows=rows.data_ptr(), counts=counts.data_ptr())
+  return source, rows, counts
+
+
+def summarize(bsuite_id: str, table: Mapping[str, Any]) -> Dict[str, Any]:
+  """Folds one id's rows (a table as `Scorer.from_rows` takes it, or `BatchedEnvironment.logged_rows()`) into its
+  score summary on the host (`bsb_score_summarize`), in the form `BatchedEnvironment.score_summary` returns:
+  a CPU float64 [B] tensor per field of `_lib.SUMMARY_FIELDS`, counts, n_points and experiment.  Raises when a
+  lane's episode column is not a prefix of the experiment's log schedule."""
+  import torch
+  lib = _lib.load()
+  source, rows, counts = _rows_source(bsuite_id, table, torch.device('cpu'))
+  batch = rows.shape[2]
+  block = torch.empty((len(_lib.SUMMARY_FIELDS), batch), dtype=torch.float64)
+  folded = torch.empty(batch, dtype=torch.int32)
+  _lib.check(lib.bsb_score_summarize(ctypes.byref(source), block.data_ptr(), folded.data_ptr()))
+  del rows, counts
+  result = {name: block[f] for f, name in enumerate(_lib.SUMMARY_FIELDS)}
+  result.update(counts=folded, n_points=int(source.n_points), experiment=experiment_of(bsuite_id))
+  return result
+
+
+_summarize = summarize        # Scorer.from_rows's `summarize` keyword hides the function's name there
 
 
 def as_numpy(result: Mapping[str, Any]) -> Dict[str, np.ndarray]:

@@ -48,7 +48,8 @@ class GraphedSweep:
 class SweepBatch:
 
   def __init__(self, bsuite_ids: Optional[Sequence[str]] = None, lanes: int = 4096, device='cuda', seed: int = 0,
-               rank: int = 0, world: int = 1, track_episodes: bool = True, ring: int = 1, record_rows: bool = False):
+               rank: int = 0, world: int = 1, track_episodes: bool = True, ring: int = 1, record_rows: bool = False,
+               track_scores: bool = False):
     import torch
     self._torch = torch
     self.bsuite_ids = list(bsuite_ids) if bsuite_ids is not None else one_per_experiment()
@@ -56,7 +57,8 @@ class SweepBatch:
     self.lanes, self.local_lanes, self.lane_offset = lanes, count, first
     self.envs = {
         bsuite_id: registry.load_from_id(bsuite_id, batch=count, device=device, seed=seed, lane_offset=first,
-                                         track_episodes=track_episodes, record_rows=record_rows)
+                                         track_episodes=track_episodes, record_rows=record_rows,
+                                         track_scores=track_scores)
         for bsuite_id in self.bsuite_ids
     }
     self._device = next(iter(self.envs.values())).device
@@ -69,6 +71,7 @@ class SweepBatch:
     self._lp = None
     self._cols = None
     self.record_rows = bool(record_rows)
+    self.track_scores = bool(track_scores)
     self._scorer = None
 
   def _ensure_buffers(self, num_steps: int):
@@ -169,12 +172,14 @@ class SweepBatch:
     return self.log_point_result(self.issue_log_point())
 
   def scores(self, out=None):
-    """Per-lane bsuite scores of this rank's lanes (`record_rows=True`): dict(scores=[23, local_lanes],
-    finished=[23, local_lanes], tags=[7, local_lanes]) on the batch's device, computed by one kernel launch on the
-    current stream from the rows recorded so far (`scoring.Scorer`).  Lanes are independent runs, so a rank needs
+    """Per-lane bsuite scores of this rank's lanes (`record_rows=True` or `track_scores=True`):
+    dict(scores=[23, local_lanes], finished=[23, local_lanes], tags=[7, local_lanes]) on the batch's device,
+    computed by one kernel launch on the current stream from the rows recorded so far, or from the score summaries
+    kept in their place (`scoring.Scorer`; both give the same bits).  Lanes are independent runs, so a rank needs
     no collective to score; a caller that wants the whole population gathers these blocks itself."""
-    if not self.record_rows:
-      raise RuntimeError('SweepBatch.scores() needs the rows of every lane: create the SweepBatch with record_rows=True')
+    if not (self.record_rows or self.track_scores):
+      raise RuntimeError('SweepBatch.scores() needs the rows or score summaries of every lane: create the SweepBatch '
+                         'with record_rows=True or track_scores=True')
     if self._scorer is None:
       from bsuite_b200 import scoring  # pylint: disable=import-outside-toplevel
       self._scorer = scoring.Scorer(self.envs)

@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define BSB_ABI_VERSION 7
+#define BSB_ABI_VERSION 8
 #define BSB_DEVICE_HOST (-1)
 #define BSB_MAX_INFO 4
 
@@ -112,7 +112,9 @@ typedef struct bsb_config {
   int32_t max_steps;
   /* mnist.py:36 (num_data = int(fraction * len(labels)), 28x28 images) */
   int32_t num_data, image_rows, image_cols;
-  int32_t reserved0;
+  /* bsb_experiment whose score summary the lanes keep (BSB_FLAG_SCORE_SUMMARY;
+   * read only with that flag, so zeroed configs are unaffected) */
+  int32_t score_experiment;
 
   double unscaled_move_cost;                         /* deep_sea.py:54 */
   double height_threshold, x_threshold, timescale,   /* cartpole.py:82-87 */
@@ -139,7 +141,9 @@ typedef struct bsb_config {
    * bsuite_num_episodes at which it writes a row.  When given (host int64
    * array; needs BSB_FLAG_TRACK_EPISODES) every lane records its own row --
    * the five Logging columns + bsuite_info() at that LAST timestep -- on the
-   * device (bsb_read_log_rows).  NULL / 0: no rows are recorded. */
+   * device (bsb_read_log_rows).  NULL / 0: no rows are recorded.
+   * BSB_FLAG_NO_LOG_ROWS keeps the schedule and the per-lane row count but no
+   * row store; BSB_FLAG_SCORE_SUMMARY folds every row into a score summary. */
   const int64_t* log_schedule;
   int64_t log_schedule_len;
 } bsb_config;
@@ -147,6 +151,15 @@ typedef struct bsb_config {
 /* bsb_config.flags */
 #define BSB_FLAG_TRACK_EPISODES 1u /* keep the Logging-wrapper accumulators
                                       (wrappers.py:85-110) per lane on device */
+/* Keep, per lane, the score summary of experiment `score_experiment` (see
+ * bsb_read_score_summary): what its scoring rule reads of the rows, folded in
+ * as each row falls due.  Needs a log schedule that is a prefix of that
+ * experiment's own schedule, BSB_FLAG_TRACK_EPISODES, and an experiment of the
+ * environment's family. */
+#define BSB_FLAG_SCORE_SUMMARY 2u
+/* With a log schedule: count the rows per lane but keep no row store (a
+ * summary-only environment does not pay for the rows). */
+#define BSB_FLAG_NO_LOG_ROWS 4u
 
 /*
  * Caller-allocated outputs of one lock-step transition.  For bsb_rollout each
@@ -279,6 +292,22 @@ int32_t bsb_sum_episode_stats_many(bsb_env* const* envs, int32_t count,
  */
 int32_t bsb_log_layout(const bsb_env* env, int32_t* n_points, int32_t* n_columns);
 int32_t bsb_read_log_rows(bsb_env* env, double* rows, int32_t* counts, void* stream);
+
+/*
+ * Per-lane score summary (BSB_FLAG_SCORE_SUMMARY): float64 [BSB_SCORE_SUMMARY_FIELDS][B], field f of lane i at
+ * summary[f * B + i], and counts int32 [B] (rows folded in so far per lane), copied into caller buffers in the
+ * environment's memory space.  The fields, over the rows of the lane so far:
+ *   last_episode, last_value   episode and value column (bsb_score_source.col_value) of the latest row
+ *   prev_episode, prev_value   the same of the row before it (NaN while there is none)
+ *   best                       running max of best_episode (cartpole, cartpole_swingup; NaN elsewhere)
+ *   first_solved               deep_sea(_stochastic): episode of the first row at or past the experiment's first
+ *                              scored episode with value / episode below its threshold (NaN until one)
+ * Every field is NaN in a lane without rows.  Because a lane's rows are always a prefix of the log schedule,
+ * these six values determine everything the experiment's scoring rule reads (bsb_scorer_* give the same bits
+ * from them as from the rows).
+ */
+#define BSB_SCORE_SUMMARY_FIELDS 6
+int32_t bsb_read_score_summary(bsb_env* env, double* summary, int32_t* counts, void* stream);
 
 /* Flat snapshot of all lane state (checkpoint/resume; absent in the reference). */
 int32_t bsb_state_bytes(const bsb_env* env, int64_t* nbytes);
@@ -446,27 +475,43 @@ const char* bsb_tag_name(int32_t tag);
  * by: noise_scale / reward_scale (the _noise / _scale experiments), height_threshold (cartpole_swingup), size
  * (deep_sea), memory_length / num_bits (memory_len / memory_size), n_distractor / chain_length (umbrella_distract /
  * umbrella_length); ignored by the other experiments.
+ *
+ * layout BSB_SCORE_ROWS (0, the value of a zeroed struct) describes rows as above.  layout BSB_SCORE_SUMMARY
+ * describes a score summary (bsb_read_score_summary, bsb_score_summarize): rows float64
+ * [BSB_SCORE_SUMMARY_FIELDS][batch], counts the rows folded in per lane, n_columns BSB_SCORE_SUMMARY_FIELDS,
+ * n_points the length of the log schedule; the col_* fields are not read.
  */
+#define BSB_SCORE_ROWS 0
+#define BSB_SCORE_SUMMARY 1
 typedef struct bsb_score_source {
   int32_t experiment;    /* bsb_experiment */
   int32_t device;        /* BSB_DEVICE_HOST or CUDA ordinal */
   int64_t batch;
   int32_t n_points, n_columns;
   int32_t col_episode, col_value, col_best;
-  int32_t reserved0;
+  int32_t layout;        /* BSB_SCORE_ROWS or BSB_SCORE_SUMMARY */
   double group_key;
   const double* rows;
   const int32_t* counts;
 } bsb_score_source;
 
 /* Fills `out` with the row store of a record-rows environment (created with a log schedule): no copy, the scorer
- * reads the environment's own rows, so the environment must outlive every scorer built from it.  Fails when the
- * environment records no rows or its family does not run `experiment`. */
+ * reads the environment's own rows, so the environment must outlive every scorer built from it.  An environment
+ * that keeps a score summary and no rows gives a BSB_SCORE_SUMMARY source over its summary instead (`experiment`
+ * must then be the one the summary is kept for).  Fails when the environment records neither, or its family does
+ * not run `experiment`. */
 int32_t bsb_score_source_from_env(const bsb_env* env, int32_t experiment, double group_key, bsb_score_source* out);
+
+/* Host only: folds caller-owned host rows (a BSB_SCORE_ROWS source on BSB_DEVICE_HOST) into a score summary,
+ * summary float64 [BSB_SCORE_SUMMARY_FIELDS][batch] and counts int32 [batch] (host buffers), with the fold the
+ * engine applies as rows fall due.  Fails when a lane's episode column is not a prefix of the experiment's log
+ * schedule (the summary is exact only for such rows). */
+int32_t bsb_score_summarize(const bsb_score_source* rows_source, double* summary, int32_t* counts);
 
 /*
  * A scorer is built once (the inputs are validated and a descriptor table is uploaded) and run many times.
  * Every source must have `batch` lanes on `device`; at most 128 sources per experiment, n_points <= 4096.
+ * Sources of both layouts may be mixed; a summary scores exactly as the rows it was folded from.
  * bsb_scorer_run writes scores float64 [BSB_NUM_EXPERIMENTS][batch], finished int32 [BSB_NUM_EXPERIMENTS][batch]
  * (the reference's _is_finished) and tags float64 [BSB_NUM_TAGS][batch], all in the memory space of `device`.
  * On CUDA it is ONE kernel launch on `stream`, with no allocation and no synchronisation, so it may be captured
